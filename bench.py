@@ -3,6 +3,8 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA engine
     python bench.py --impl reference --gpus N --steps K ...  # the CPU arm (oracle; see below)
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's results (dump_outputs):
+                                                             # rank 0's windows only under --gpus > 1; not with --inproc
 
 Workload (BASELINE.json configs[4], the configuration the metric is quoted on, per GPU):
 Whisper large-v3 (128 mel), greedy, batch 64, 128 x 30 s windows per GPU per step (1024 windows
@@ -91,6 +93,54 @@ def window_clip(info, index):
     return synth_audio.keyed_clip(info["keyed"], sym, seed=5000 + index), gen_model.keyed_expected_tokens(info, sym)
 
 
+DUMP_LIMIT = 64 << 20
+TOKEN_FLOATS = ("p", "plog", "pt", "ptsum", "vlen")
+
+
+def dump_outputs(out_dir, windows, results):
+    """Writes what a caller received from the last timed step, one array per field as out_dir/<name>.npy, so that
+    two builds can be compared output for output: per window (`windows[i]` is result i's index in the workload) its
+    language and decoder step count, per segment its bounds, per token its id, timestamp token, probabilities and
+    times, each row tagged with its window (and segment). Token probabilities are float32 as computed; integers are
+    stored exactly as float64. Above DUMP_LIMIT bytes in all, a seeded sample of whole windows is written."""
+    def tables(sel):
+        t = {k: [] for k in ("window_index", "window_lang_id", "window_n_decode_steps", "segment_window",
+                             "segment_t0", "segment_t1", "segment_speaker_turn_next", "token_window", "token_segment",
+                             "token_id", "token_tid", "token_t0", "token_t1") + tuple("token_" + f for f in TOKEN_FLOATS)}
+        for i in sel:
+            w, r = windows[i], results[i]
+            t["window_index"].append(w)
+            t["window_lang_id"].append(r["lang_id"])
+            t["window_n_decode_steps"].append(r["n_decode_steps"])
+            for s, seg in enumerate(r["segments"]):
+                t["segment_window"].append(w)
+                for k in ("t0", "t1", "speaker_turn_next"):
+                    t["segment_" + k].append(seg[k])
+                for tok in seg["tokens"]:
+                    t["token_window"].append(w)
+                    t["token_segment"].append(s)
+                    for k in ("id", "tid", "t0", "t1") + TOKEN_FLOATS:
+                        t["token_" + k].append(tok[k])
+        floats = {"token_" + f for f in TOKEN_FLOATS}
+        return {k: np.asarray(v, np.float32 if k in floats else np.float64) for k, v in t.items()}
+
+    size = [sum(a.nbytes for a in tables([i]).values()) for i in range(len(results))]
+    sel = list(range(len(results)))
+    if sum(size) > DUMP_LIMIT:
+        sel, total = [], 0
+        for i in np.random.default_rng(0).permutation(len(results)):
+            if total + size[i] > DUMP_LIMIT:
+                break
+            sel.append(int(i))
+            total += size[i]
+        sel.sort()
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in tables(sel).items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+    print("bench.py: outputs of %d of %d windows of the last timed step written to %s" % (len(sel), len(results), out_dir),
+          file=sys.stderr)
+
+
 class ClockSampler:
     """nvidia-smi clocks / throttle reasons DURING the timed region (B200_PROFILING.md recipe)."""
     Q = ("clocks.sm,clocks.max.sm,power.draw,clocks_event_reasons.hw_slowdown,"
@@ -146,6 +196,8 @@ def run_reference(args, rank, world):
         dt = time.perf_counter() - t0
         if s >= args.warmup:
             times.append(dt)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, [s], [r])
     total = sum(times)
     val = 30.0 * len(times) / total
     line = dict(
@@ -203,7 +255,14 @@ def main():
                     help="(default) also measure the reference-facing class: caller threads on SttEngine::transcribe_pcm16 "
                          "with pageable vectors (host/stt_cli bench mode) -> e2e_facade")
     ap.add_argument("--no-facade", dest="facade", action="store_false")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the results of the last timed step (rank 0's windows) as "
+                         "DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.inproc > 0:
+        ap.error("--dump-outputs is not supported with --inproc")
     cfg = dict(CONFIGS[args.config])
     if args.model:
         cfg["model"] = args.model
@@ -309,7 +368,9 @@ def main():
     parity = dict(windows=0, token_identical_to_expected=0, distinct_transcripts=0)
     seen, got_ids = set(), {}
 
-    def step(which, check=False):
+    def step(which, check=False, keep=None):
+        """One pass over the rank's windows. keep: a list that takes (window, result handle) pairs instead of
+        freeing the results, for reading after the timed region."""
         n_tok = 0
         for g in groups:
             res = eng.full_batch_ptrs(g[which], g["lens"], g["n"], params_by_lang[g["lang"]], languages=g["langs"])
@@ -326,12 +387,15 @@ def main():
                     parity["token_identical_to_expected"] += int(ids[:k] == want_ids[w][:k] and (k < len(want_ids[w]) or ids == want_ids[w]))
                     seen.add(tuple(ids))
                     got_ids[w] = ids
-                L.sw_result_free(r)
+                if keep is not None:
+                    keep.append((w, r))
+                else:
+                    L.sw_result_free(r)
         return n_tok
 
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
 
-    def timed(which, k):
+    def timed(which, k, keep=None):
         """K steps between a barrier + device synchronize on both sides, timed with two CUDA events. The device
         is idle when the first is recorded (synchronize just before) and every step call returns only after
         its last kernel and read-back have completed (the sequencer reads the picks of every decoder step), so
@@ -341,8 +405,8 @@ def main():
         t0 = time.perf_counter()
         ev0.record()
         n_tok = 0
-        for _ in range(k):
-            n_tok += step(which)
+        for i in range(k):
+            n_tok += step(which, keep=keep if i == k - 1 else None)
         ev1.record()
         torch.cuda.synchronize()
         wall = time.perf_counter() - t0
@@ -359,11 +423,14 @@ def main():
     clocks = ClockSampler(local_rank)
     if rank == 0:  # one sampler per job: the line reports rank 0's GPU, and nvidia-smi polling is not free
         clocks.start()
-    dt, n_tok, wall = timed("dev", args.steps)
+    last = [] if args.dump_outputs and rank == 0 else None
+    dt, n_tok, wall = timed("dev", args.steps, keep=last)
     st = eng.stats(reset=True)
     dt_e2e, _, wall_e2e = timed("host", args.steps)
     st_e2e = eng.stats(reset=True)
     clk = clocks.stop()
+    if last is not None:
+        dump_outputs(args.dump_outputs, [mine[w] for w, _ in last], [eng._collect(r) for _, r in last])
 
     audio_local = float(sum(n_samp)) / 16000.0
     audio_all = audio_local

@@ -1,9 +1,10 @@
 """CPU tests pinning the oracle's logit rules and greedy sequencing against HuggingFace's independent
 implementation of the same OpenAI rules (generation/logits_process.py:1812-2046 and
 WhisperForConditionalGeneration.generate). The fixtures are produced by HF code alone
-(tests/golden/make_rules_golden.py -> golden/rules_hf.npz); when `transformers` is importable the HF side is
-also re-run live. The two intentional whisper.cpp-vs-OpenAI differences (D1, D2: see make_rules_golden.py)
-are asserted explicitly instead of being tolerated."""
+(tests/golden/make_rules_golden.py -> golden/rules_hf.npz, tests/golden/make_hf_cases_golden.py ->
+golden/hf_cases.npz); when `transformers` is importable the HF side is also re-run live. The two intentional
+whisper.cpp-vs-OpenAI differences (D1, D2: see make_rules_golden.py) are asserted explicitly instead of being
+tolerated."""
 import ast
 import os
 import sys
@@ -16,6 +17,7 @@ from tools import ggml_io, synth_audio
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(HERE, "golden"))
+import make_hf_cases_golden as mhc  # noqa: E402
 import make_rules_golden as mrg  # noqa: E402
 
 
@@ -24,10 +26,24 @@ def ctx(ora):
     g = np.load(os.path.join(HERE, "golden", "rules_hf.npz"))
     args = ast.literal_eval(str(g["model_args"]))
     assert args == mrg.MODEL_ARGS
+    hf = np.load(os.path.join(HERE, "golden", "hf_cases.npz"))
+    assert ast.literal_eval(str(hf["model_args"])) == mrg.MODEL_ARGS
     path, info = model_file(args["size"], seed=args["seed"], script_len=args["script_len"], keyed=args["keyed"])
     hp, _, vocab, _ = ggml_io.read_ggml(path)
     o = ora.Oracle(path)
-    return dict(g=g, path=path, info=info, sp=info["special"], vocab=vocab, n_vocab=hp["n_vocab"], o=o)
+    return dict(g=g, hf=hf, path=path, info=info, sp=info["special"], vocab=vocab, n_vocab=hp["n_vocab"], o=o)
+
+
+def hf_masks(ctx, key, cs):
+    """HF's -inf masks for the (history, logits) cases `cs`: as stored in golden/hf_cases.npz[key] and, when
+    transformers is importable, recomputed live; the oracle is held to each of them."""
+    out = [np.unpackbits(ctx["hf"][key], axis=1)[:, : ctx["n_vocab"]].astype(bool)]
+    assert len(out[0]) == len(cs)
+    try:
+        import transformers  # noqa: F401
+    except ImportError:
+        return out
+    return out + [mhc.hf_case_masks(ctx["sp"], ctx["vocab"], cs)]
 
 
 def decoder_state(hist, beg):
@@ -90,30 +106,24 @@ def test_masks_match_hf_golden(ctx):
 
 
 def test_masks_match_hf_live(ctx):
-    pytest.importorskip("transformers")
     sp = ctx["sp"]
-    prompt = [sp["sot"], sp["sot"] + 1, sp["transcribe"]]
-    procs = mrg.hf_processors(sp, ctx["vocab"], len(prompt))
-    cs = mrg.cases(sp, ctx["n_vocab"], len(ctx["vocab"]) - 1, seed=77, n=48)
-    for hist, logits in cs:
-        want, _ = mrg.hf_mask(procs, prompt, hist, logits)
+    cs = mrg.cases(sp, ctx["n_vocab"], len(ctx["vocab"]) - 1, seed=mhc.LIVE_SEED, n=mhc.N_LIVE)
+    hf = hf_masks(ctx, "live_masks", cs)
+    for i, (hist, logits) in enumerate(cs):
         got, _, _, _ = oracle_mask(ctx, hist, logits)
-        assert np.array_equal(got, want)
+        for want in hf:
+            assert np.array_equal(got, want[i])
 
 
 def test_named_difference_d1_initial_text_not_forced(ctx):
     """OpenAI/HF force a timestamp at the first sampled position; whisper.cpp only through the mass rule."""
-    pytest.importorskip("transformers")
     sp, n = ctx["sp"], ctx["n_vocab"]
-    prompt = [sp["sot"], sp["sot"] + 1, sp["transcribe"]]
-    procs = mrg.hf_processors(sp, ctx["vocab"], len(prompt))
-    logits = np.random.default_rng(1).normal(0, 1, n).astype(np.float32)
-    logits[2000] += 30.0                                   # a text token dominates
-    want, _ = mrg.hf_mask(procs, prompt, [], logits)
-    got, _, _, _ = oracle_mask(ctx, [], logits)
+    cs = mhc.d1_cases(sp, n)                               # no history; a text token dominates
+    got, _, _, _ = oracle_mask(ctx, *cs[0])
     beg = sp["beg"]
-    assert want[:beg].all() and not got[2000]              # HF: no text at all; whisper.cpp: text survives
-    assert np.array_equal(got[beg:], want[beg:])           # same max_initial_ts window (<= 1.00 s)
+    for want, in hf_masks(ctx, "d1_masks", cs):
+        assert want[:beg].all() and not got[2000]          # HF: no text at all; whisper.cpp: text survives
+        assert np.array_equal(got[beg:], want[beg:])       # same max_initial_ts window (<= 1.00 s)
     static = np.zeros(n, bool)
     static[mrg.static_suppress_ids(ctx["vocab"], sp)] = True
     static[[sp["not_"], sp["eot"], mrg.space_id(ctx["vocab"])]] = True
@@ -122,18 +132,15 @@ def test_named_difference_d1_initial_text_not_forced(ctx):
 
 def test_named_difference_d2_equal_timestamp_allowed(ctx):
     """After text that follows a timestamp, HF forbids timestamps <= the last one; whisper.cpp only < it."""
-    pytest.importorskip("transformers")
     sp, n = ctx["sp"], ctx["n_vocab"]
     beg = sp["beg"]
-    prompt = [sp["sot"], sp["sot"] + 1, sp["transcribe"]]
-    procs = mrg.hf_processors(sp, ctx["vocab"], len(prompt))
-    logits = np.random.default_rng(2).normal(0, 1, n).astype(np.float32)
-    for hist in ([beg, 1000, beg + 40, beg + 40, 1001], [beg, 1000, 1001]):
-        want, _ = mrg.hf_mask(procs, prompt, hist, logits)
-        got, _, _, _ = oracle_mask(ctx, hist, logits)
-        last = max(t for t in hist if t >= beg)
-        diff = np.flatnonzero(got != want)
-        assert diff.tolist() == [last] and want[last] and not got[last]
+    cs = mhc.d2_cases(sp, n)
+    for masks in hf_masks(ctx, "d2_masks", cs):
+        for (hist, logits), want in zip(cs, masks):
+            got, _, _, _ = oracle_mask(ctx, hist, logits)
+            last = max(t for t in hist if t >= beg)
+            diff = np.flatnonzero(got != want)
+            assert diff.tolist() == [last] and want[last] and not got[last]
 
 
 def test_greedy_sequence_matches_hf_generate_golden(ctx, ora):
