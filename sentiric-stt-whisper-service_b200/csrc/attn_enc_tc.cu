@@ -13,9 +13,7 @@
 // its shadow and meet it again at pass 2 of tile j+1, which needs P's columns back.
 // Two CTAs share an SM (112 KB smem, 256 TMEM columns each): one CTA's softmax overlaps the other's
 // MMAs. Replaces ggml's flash_attn_ext in whisper_encode_internal (SURVEY.md A.4); generation 1
-// (attn_enc.cu, mma.sync) reached 298 TFLOP/s and was 35 % of the encoder time.
-#include <stdlib.h>
-
+// (mma.sync) reached 298 TFLOP/s and was 35 % of the encoder time.
 #include "common.cuh"
 #include "gemm.cuh"
 #include "kernels.cuh"
@@ -35,14 +33,9 @@ constexpr int ATT_THREADS = 320;       // warp 0: TMA, warp 1: TMEM + MMA issue,
 // over the scores it came from and double-buffered O instead: P V(j) then had to be issued BEFORE S(j+1) and sat
 // on the serial chain; 1.44 vs 1.37 ms per layer for 64 windows.)
 constexpr int TMEM_COLS = 256, TM_P = 128, TM_O = 192;
-// Measured and rejected (round 2, profiles/r2_attn_exp2_poly.txt): with every third exponential on the FMA pipe the
-// encoder went from 2.65 to 2.73 ms per window - pass 2 is bound by issue slots (ex2 + ffma + cvt + the tcgen05.ld/st
-// traffic of 256 softmax threads), not by the MUFU unit alone, and the nine extra FMA/ALU instructions per element
-// cost more than the ex2 they replace. Kept behind -DSW_ATT_POLY=1.
-#ifndef SW_ATT_POLY
-#define SW_ATT_POLY 0
-#endif
-constexpr bool ATT_POLY = SW_ATT_POLY != 0;
+// Measured and rejected (round 2, DESIGN.md §4 "Where the time is now"): a third of the exponentials on the FMA pipe
+// (slower: pass 2 is bound by issue slots, not by the MUFU unit alone) and a one-pass softmax shifted by the maximum
+// of the previous tiles (encoder time unchanged: the two CTAs of an SM are bound by the exponentials they share).
 
 // MN-major 128B-swizzled operand (the V tile: rows = keys (K), 64 dims (MN) contiguous per row):
 // canonical layout ((8,n),(8,k)):((1,LBO),(8,SBO)) in 16-byte units -> SBO = 1024 B between 8-key groups
@@ -62,31 +55,8 @@ __device__ __forceinline__ float fast_exp2(float x) {
   return y;
 }
 
-// 2^x for x <= 0 on the FMA / ALU pipes (Cody-Waite split + cubic), for a share of the softmax exponentials: the
-// MUFU unit evaluates 16 ex2 per clock and SM, and pass 2 of a key tile needs 16 384 per CTA - the pipe that
-// bounds this kernel (DESIGN.md). round(x) comes out of the magic-number add (1.5 * 2^23), the cubic covers
-// [-0.5, 0.5] with a relative error of 6e-4 (P is rounded to bf16, 2e-3, right after), and the integer part goes
-// into the exponent field with one shift and one add.
-__device__ __forceinline__ float exp2_fma(float x) {
-  x = fmaxf(x, -125.f);
-  const float t = x + 12582912.f;
-  const float f = x - (t - 12582912.f);
-  float p = fmaf(f, 0.05550411f, 0.24022651f);
-  p = fmaf(p, f, 0.69314718f);
-  p = fmaf(p, f, 1.0f);
-  return __int_as_float(__float_as_int(p) + (__float_as_int(t) << 23));
-}
-
-// LAGGED: the softmax of key tile j >= 1 is shifted by the running maximum of the tiles BEFORE it instead of its own
-// (any shift is a valid softmax shift as long as nothing overflows: P is a floating-point format, so its relative
-// precision does not depend on the shift), which removes the separate maximum pass - and the second tcgen05.ld of the
-// scores - from every tile but the first: the maximum of tile j is gathered inside the exponential pass and only
-// moves the shift of tile j + 1. A row whose tile maximum exceeds the shift by more than 2^60 recomputes its
-// probabilities with the new maximum (warp-uniform decision; both threads of a row take it together).
-template <bool LAGGED>
 __global__ void __launch_bounds__(ATT_THREADS, 2)
-encoder_attention_tc_kernel(const __grid_constant__ CUtensorMap map_qkv, bf16* __restrict__ out, int T, int d,
-                            long long* __restrict__ trace) {  // trace: development timestamps (SW_ATTN_TRACE) or null
+encoder_attention_tc_kernel(const __grid_constant__ CUtensorMap map_qkv, bf16* __restrict__ out, int T, int d) {
   extern __shared__ __align__(1024) uint8_t smem[];
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem + SM_BARS);
   uint64_t* q_full = bars;
@@ -103,13 +73,6 @@ encoder_attention_tc_kernel(const __grid_constant__ CUtensorMap map_qkv, bf16* _
   const int warp = __shfl_sync(0xffffffffu, threadIdx.x >> 5, 0), lane = threadIdx.x & 31;  // warp: provably uniform
   const int q0 = qt * TQ;
   const int n_tiles = (T + TK - 1) / TK;
-  // development: clock64 stamps of one CTA in the middle of the grid: [role 0 = softmax warp 2 lane 0,
-  // role 1 = MMA thread][tile][event]
-  const bool tr = trace && blockIdx.x == 5 && blockIdx.y == 7 && blockIdx.z == (gridDim.z >> 1);
-#define ATT_TRACE(role, tile, ev)                                                        \
-  do {                                                                                   \
-    if (tr) trace[((role) * 16 + (tile)) * 8 + (ev)] = clock64();                        \
-  } while (0)
   const int row_base = w * T;
 
   if (threadIdx.x == 0) {
@@ -177,14 +140,11 @@ encoder_attention_tc_kernel(const __grid_constant__ CUtensorMap map_qkv, bf16* _
         const int s = j & 1;
         const uint32_t ph = (j >> 1) & 1;
         const uint32_t sv = smem_u32(smem + SM_V + s * TILE_BYTES);
-        ATT_TRACE(1, j, 0);
         mbar_wait(p_ready, j & 1);
         tc_fence_after();
-        ATT_TRACE(1, j, 1);
         // every softmax thread is past its last read of S(j): the next scores go first, so that the serial chain
         // of a key tile is softmax -> S(j+1) and P V(j) runs in its shadow
         if (j + 1 < n_tiles) issue_s(j + 1);
-        ATT_TRACE(1, j, 2);
         mbar_wait(o_free, j & 1);
         tc_fence_after();
         mbar_wait(&v_full[s], ph);
@@ -197,7 +157,6 @@ encoder_attention_tc_kernel(const __grid_constant__ CUtensorMap map_qkv, bf16* _
         }
         umma_commit(o_full);
         umma_commit(&kv_empty[s]);
-        ATT_TRACE(1, j, 3);
       }
     }
   } else {
@@ -228,117 +187,91 @@ encoder_attention_tc_kernel(const __grid_constant__ CUtensorMap map_qkv, bf16* _
     };
     const uint32_t s_addr = tmem + lane_addr + half * 64;
     const uint32_t p_addr = tmem + lane_addr + TM_P + half * 32;  // this thread's 64 probabilities: 32 packed columns
-    float shift_prev = 0.f;  // LAGGED: the shift the previous tile's probabilities were computed with
     for (int j = 0; j < n_tiles; ++j) {
       const int valid = min(TK, T - j * TK);
       mbar_wait(s_full, j & 1);
       tc_fence_after();
-      if (warp == 2 && lane == 0) ATT_TRACE(0, j, 0);
+      // ---- pass 1: the maximum of this thread's 64 scores
+      float mx = -INFINITY;
+#pragma unroll
+      for (int cc = 0; cc < 2; ++cc) {
+        const int c = half * 2 + cc;
+        uint32_t r[32];
+        tmem_ld_32x32b_x32(s_addr + cc * 32, r);
+        tmem_ld_wait(r);
+        if (c * 32 + 32 <= valid) {
+#pragma unroll
+          for (int i = 0; i < 32; ++i) mx = fmaxf(mx, __uint_as_float(r[i]));
+        } else {
+#pragma unroll
+          for (int i = 0; i < 32; ++i)
+            if (c * 32 + i < valid) mx = fmaxf(mx, __uint_as_float(r[i]));
+        }
+      }
       // the row maximum of this thread's 64 scores meets its partner's in shared memory. The partner's previous read
       // of this slot happened before it arrived on p_ready for tile j-1, and S_j (whose completion we just waited
       // for) was issued after all eight warps had arrived: no race. Exchanged as bf16 ROUNDED UP (both threads of
       // the row must use the same value; 512 bytes instead of 1 KB keep two CTAs on an SM).
-      auto exchange_max = [&](float mx) {
+      {
         const uint32_t u = __float_as_uint(mx);
         uint32_t t = u & 0xffff0000u;
         if (t != u && !(u >> 31)) t += 0x10000u;
         mx = __uint_as_float(t);
         xch[half * 128 + row] = static_cast<uint16_t>(t >> 16);
         asm volatile("bar.sync 1, 256;" ::: "memory");
-        return fmaxf(mx, __uint_as_float(static_cast<uint32_t>(xch[(half ^ 1) * 128 + row]) << 16));
-      };
-      // one sweep over this thread's 64 scores: P = exp2(S * sc - shift) -> bf16 -> tensor memory (the A operand of
-      // P V, TS form); returns the row-sum share and the raw maximum of the scores
-      float lsum = 0.f, mx = -INFINITY;
-      auto sweep = [&](float shift, bool want_p) {
-        lsum = 0.f;
-        mx = -INFINITY;
-#pragma unroll
-        for (int cc = 0; cc < 2; ++cc) {
-          const int c = half * 2 + cc;
-          uint32_t r[32];
-          tmem_ld_32x32b_x32(s_addr + cc * 32, r);
-          tmem_ld_wait(r);
-          const bool full = c * 32 + 32 <= valid;
-          if (full) {
-#pragma unroll
-            for (int i = 0; i < 32; ++i) mx = fmaxf(mx, __uint_as_float(r[i]));
-          } else {
-#pragma unroll
-            for (int i = 0; i < 32; ++i)
-              if (c * 32 + i < valid) mx = fmaxf(mx, __uint_as_float(r[i]));
-          }
-          if (!want_p) continue;
-          uint32_t pk[16];
-          if (full) {  // no masking
-#pragma unroll
-            for (int i = 0; i < 16; ++i) {
-              const float p0 = fast_exp2(__uint_as_float(r[2 * i]) * sc - shift);
-              // every third exponential on the FMA pipe (exp2_fma): MUFU and FMA then finish together
-              const float x1 = __uint_as_float(r[2 * i + 1]) * sc - shift;
-              const float p1 = (ATT_POLY && i % 3 != 2) ? exp2_fma(x1) : fast_exp2(x1);
-              lsum += p0 + p1;
-              pk[i] = pack_bf16x2(p0, p1);
-            }
-          } else {
-#pragma unroll
-            for (int i = 0; i < 16; ++i) {
-              float p0 = fast_exp2(__uint_as_float(r[2 * i]) * sc - shift);
-              float p1 = fast_exp2(__uint_as_float(r[2 * i + 1]) * sc - shift);
-              if (c * 32 + 2 * i >= valid) p0 = 0.f;
-              if (c * 32 + 2 * i + 1 >= valid) p1 = 0.f;
-              lsum += p0 + p1;
-              pk[i] = pack_bf16x2(p0, p1);
-            }
-          }
-          // P's columns are free once P V(j-1) has completed. It was queued behind S(j), whose completion started
-          // this sweep; by the time the first 32 probabilities exist it is long done, so the wait sits here and not in
-          // front of the sweep
-          if (cc == 0 && j > 0) {
-            mbar_wait(o_full, (j - 1) & 1);
-            tc_fence_after();
-          }
-          // 32 keys = 16 packed columns of this row, over scores this thread has already consumed
-          tmem_st_32x32b_x16(p_addr + cc * 16, pk);
-        }
-      };
-      float shift;  // of this tile's probabilities
-      if (!LAGGED || j == 0) {
-        // ---- two passes: the tile's own maximum first
-        sweep(0.f, false);
-        if (warp == 2 && lane == 0) ATT_TRACE(0, j, 1);
-        mx = exchange_max(mx);
-        if (warp == 2 && lane == 0) ATT_TRACE(0, j, 2);
-        m = fmaxf(m, mx * sc);
-        shift = m;
-        sweep(shift, true);
-      } else {
-        // ---- one pass, shifted by the maximum of the tiles before this one
-        shift = m;
-        sweep(shift, true);
-        if (warp == 2 && lane == 0) ATT_TRACE(0, j, 1);
-        mx = exchange_max(mx);
-        if (warp == 2 && lane == 0) ATT_TRACE(0, j, 2);
-        m = fmaxf(m, mx * sc);
-        if (__any_sync(0xffffffffu, m - shift > 60.f)) {  // the same 32 rows vote in both warps of a row
-          shift = m;
-          sweep(shift, true);
-        }
+        mx = fmaxf(mx, __uint_as_float(static_cast<uint32_t>(xch[(half ^ 1) * 128 + row]) << 16));
       }
-      const float alpha = j == 0 ? 1.f : fast_exp2(shift_prev - shift);
-      shift_prev = shift;
+      const float m_prev = m;
+      m = fmaxf(m, mx * sc);
+      // ---- pass 2: P = exp2(S * sc - m) -> bf16 -> tensor memory (the A operand of P V, TS form), and this
+      // thread's share of the row sum
+      float lsum = 0.f;
+#pragma unroll
+      for (int cc = 0; cc < 2; ++cc) {
+        const int c = half * 2 + cc;
+        uint32_t r[32];
+        tmem_ld_32x32b_x32(s_addr + cc * 32, r);
+        tmem_ld_wait(r);
+        uint32_t pk[16];
+        if (c * 32 + 32 <= valid) {  // no masking
+#pragma unroll
+          for (int i = 0; i < 16; ++i) {
+            const float p0 = fast_exp2(__uint_as_float(r[2 * i]) * sc - m);
+            const float p1 = fast_exp2(__uint_as_float(r[2 * i + 1]) * sc - m);
+            lsum += p0 + p1;
+            pk[i] = pack_bf16x2(p0, p1);
+          }
+        } else {
+#pragma unroll
+          for (int i = 0; i < 16; ++i) {
+            float p0 = fast_exp2(__uint_as_float(r[2 * i]) * sc - m);
+            float p1 = fast_exp2(__uint_as_float(r[2 * i + 1]) * sc - m);
+            if (c * 32 + 2 * i >= valid) p0 = 0.f;
+            if (c * 32 + 2 * i + 1 >= valid) p1 = 0.f;
+            lsum += p0 + p1;
+            pk[i] = pack_bf16x2(p0, p1);
+          }
+        }
+        // P's columns are free once P V(j-1) has completed. It was queued behind S(j), whose completion started
+        // this pass; by the time the first 32 probabilities exist it is long done, so the wait sits here and not in
+        // front of the pass
+        if (cc == 0 && j > 0) {
+          mbar_wait(o_full, (j - 1) & 1);
+          tc_fence_after();
+        }
+        // 32 keys = 16 packed columns of this row, over scores this thread has already consumed
+        tmem_st_32x32b_x16(p_addr + cc * 16, pk);
+      }
+      const float alpha = j == 0 ? 1.f : fast_exp2(m_prev - m);
       l = l * alpha + lsum;  // this thread's half of the row sum (same alpha in both halves)
-      if (warp == 2 && lane == 0) ATT_TRACE(0, j, 3);
       tmem_st_wait();
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(p_ready);
-      if (warp == 2 && lane == 0) ATT_TRACE(0, j, 4);
       // fold the PREVIOUS tile's O while the tensor core works on this tile's P V and the next Q K^T
       if (j > 0) fold_o(j - 1, alpha_prev);
       __syncwarp();  // O is free: P V(j), queued behind S(j+1), may overwrite it
       if (lane == 0) mbar_arrive(o_free);
-      if (warp == 2 && lane == 0) ATT_TRACE(0, j, 5);
       alpha_prev = alpha;
     }
     fold_o(n_tiles - 1, alpha_prev);
@@ -377,41 +310,11 @@ int encoder_attention_tc(const bf16* qkv, bf16* out, int n_win, int T, int d, in
   if (n_win <= 0) return 0;
   SW_CHECK(d == n_head * DH, "encoder_attention: head dim must be 64 (d=%d heads=%d)", d, n_head);
   static SmemOptIn opt_in;  // per device (host_common.h)
-  static SmemOptIn opt_in2;
-  SW_CUDA_CHECK(opt_in.ensure(encoder_attention_tc_kernel<true>, ATT_SMEM));
-  SW_CUDA_CHECK(opt_in2.ensure(encoder_attention_tc_kernel<false>, ATT_SMEM));
-  // development switch: SW_ATT_LAGGED=1 selects the one-pass softmax with the lagged shift. Measured (round 2, ABAB on
-  // one box, profiles/r2_attn_lagged_max.txt): parity green, encoder time unchanged (344.5 / 344.0 vs 344.4 / 349.6 ms
-  // per 128 windows) - removing the maximum pass does not shorten a key tile because the SM's two CTAs are bound by
-  // the exponentials they share, not by the instructions around them. The two-pass kernel stays the default.
-  static const bool lagged = getenv("SW_ATT_LAGGED") && atoi(getenv("SW_ATT_LAGGED")) == 1;
+  SW_CUDA_CHECK(opt_in.ensure(encoder_attention_tc_kernel, ATT_SMEM));
   CUtensorMap map;
   if (make_tma_map_2d_bf16(&map, qkv, 3 * (int64_t)d, (int64_t)n_win * T, 3 * (int64_t)d, 64, 128)) return -1;
   dim3 grid((T + TQ - 1) / TQ, n_head, n_win);
-  static int trace_left = getenv("SW_ATTN_TRACE") ? 1 : 0;  // development: time one CTA of one launch
-  long long* d_trace = nullptr;
-  if (trace_left > 0 && n_win >= 8) {
-    cudaMalloc(&d_trace, 2 * 16 * 8 * sizeof(long long));
-    cudaMemset(d_trace, 0, 2 * 16 * 8 * sizeof(long long));
-  }
-  if (lagged) encoder_attention_tc_kernel<true><<<grid, ATT_THREADS, ATT_SMEM, stream>>>(map, out, T, d, d_trace);
-  else encoder_attention_tc_kernel<false><<<grid, ATT_THREADS, ATT_SMEM, stream>>>(map, out, T, d, d_trace);
-  if (d_trace) {
-    trace_left = 0;
-    long long h[2 * 16 * 8];
-    cudaStreamSynchronize(stream);
-    cudaMemcpy(h, d_trace, sizeof(h), cudaMemcpyDeviceToHost);
-    cudaFree(d_trace);
-    const long long t00 = h[0];
-    for (int j = 0; j < 12; ++j) {
-      const long long* a = h + j * 8;
-      const long long* b = h + (16 + j) * 8;
-      fprintf(stderr, "[attn trace] tile %2d softmax: S seen %7lld | pass1 %5lld | bar %5lld | pass2 %5lld | fence+arrive %5lld | fold %5lld || "
-                      "mma: wait P from %7lld, seen %7lld, PV issued +%4lld, S(j+1) issued +%4lld\n",
-              j, a[0] - t00, a[1] - a[0], a[2] - a[1], a[3] - a[2], a[4] - a[3], a[5] - a[4], b[0] - t00, b[1] - t00,
-              b[2] - b[1], b[3] - b[2]);
-    }
-  }
+  encoder_attention_tc_kernel<<<grid, ATT_THREADS, ATT_SMEM, stream>>>(map, out, T, d);
   SW_CUDA_CHECK(cudaGetLastError());
   return 0;
 }

@@ -40,26 +40,15 @@ sw_ctx* sw_ctx_create(const char* path, const sw_ctx_params* params) {
     set_last_error("null model path");
     return nullptr;
   }
-  // Lane mode "interleaved" (SW_INTERLEAVE=1, development): instead of n independent lanes (threads, streams,
-  // graphs), ONE engine takes n_lanes x max_batch windows per pass and cuts every decoder step into two halves
-  // whose chains and cross attentions alternate inside one graph (engine.cu::enqueue_decode_step)
-  sw_ctx_params pi = params ? *params : sw_ctx_default_params();
-  const char* il = getenv("SW_INTERLEAVE");
-  const bool interleave = il && atoi(il) == 1 && pi.n_lanes != 1;
-  if (interleave) {
-    pi.max_batch = 2 * (pi.max_batch > 0 ? pi.max_batch : 64);
-    pi.n_lanes = 1;
-    pi.reserved[0] = 1;
-  }
+  const sw_ctx_params pi = params ? *params : sw_ctx_default_params();
   Engine* e = sw::engine_create(path, &pi);
   if (!e) return nullptr;
   if (const char* v = getenv("SW_XA_CTAS")) e->xa_max_ctas = atoi(v);  // development: cap also without lanes
   sw_ctx* c = new sw_ctx();
   c->e = e;
-  params = &pi;
   // further lanes (sw_ctx_params.n_lanes; SW_LANES overrides for experiments). Auto: a second lane when
   // its buffers fit twice over in what is left of the device memory.
-  int want = params ? params->n_lanes : 0;
+  int want = pi.n_lanes;
   if (const char* v = getenv("SW_LANES")) want = atoi(v);
   if (want <= 0) {
     size_t free_b = 0, total_b = 0;

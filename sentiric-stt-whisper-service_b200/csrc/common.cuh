@@ -184,25 +184,12 @@ __device__ __forceinline__ void tma_load_3d(void* smem_dst, const void* map, uin
       : "memory");
 }
 
-// L2 eviction policies for streamed operands: data that is read once (the cross-KV cache) should not push
+// L2 eviction policy for streamed operands: data that is read once (the cross-KV cache) should not push
 // out what another kernel re-reads soon (decoder weights, shared by the lanes).
 __device__ __forceinline__ uint64_t l2_policy_evict_first() {
   uint64_t p;
   asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(p));
   return p;
-}
-__device__ __forceinline__ uint64_t l2_policy_evict_last() {
-  uint64_t p;
-  asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(p));
-  return p;
-}
-__device__ __forceinline__ void tma_load_2d_hint(void* smem_dst, const void* map, uint64_t* bar, int c0, int c1,
-                                                 uint64_t policy) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint "
-      "[%0], [%1, {%3, %4}], [%2], %5;" ::"r"(smem_u32(smem_dst)),
-      "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "l"(policy)
-      : "memory");
 }
 __device__ __forceinline__ void tma_load_3d_hint(void* smem_dst, const void* map, uint64_t* bar, int c0, int c1, int c2,
                                                  uint64_t policy) {

@@ -574,12 +574,9 @@ static int launch_process_logits(const float* logits, int64_t ld, const LogitRow
 int process_logits_pick(const float* logits, int64_t ld, const LogitRow* d_rows, int R,
                         const LogitCfg& cfg, PickOut* d_out, cudaStream_t stream) {
   if (R <= 0) return 0;
-  // CTAs per row: as many as keep the launch inside one wave (a CTA is 1024 threads x 64 registers = one SM);
-  // SW_LP_CLUSTER forces 1 / 2 / 4 (development)
-  static const int forced = getenv("SW_LP_CLUSTER") ? atoi(getenv("SW_LP_CLUSTER")) : 0;
+  // CTAs per row: as many as keep the launch inside one wave (a CTA is 1024 threads x 64 registers = one SM)
   const int sms = device_sm_count();
-  int cl = R * 4 <= sms ? 4 : R * 2 <= sms ? 2 : 1;
-  if (forced == 1 || forced == 2 || forced == 4) cl = forced;
+  const int cl = R * 4 <= sms ? 4 : R * 2 <= sms ? 2 : 1;
   if (cl == 4) return launch_process_logits<4>(logits, ld, d_rows, R, cfg, d_out, stream);
   if (cl == 2) return launch_process_logits<2>(logits, ld, d_rows, R, cfg, d_out, stream);
   return launch_process_logits<1>(logits, ld, d_rows, R, cfg, d_out, stream);

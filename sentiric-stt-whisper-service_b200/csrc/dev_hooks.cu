@@ -117,9 +117,12 @@ int sw_dev_skinny_gemm_k(int kernel, const void* dX, const void* dW, int R, int 
     if (split <= 0) split = sw::skinny_tc_split_for(N, K);
     return sw::skinny_gemm_tc(X, K, W, R, N, K, d_bias, gelu, static_cast<sw::bf16*>(d_out), N, d_partial, split, st);
   }
-  if (split <= 0) split = kernel == 1 ? sw::skinny_mma_split_for(N, K) : sw::skinny_split_for(N, K);
-  return sw::skinny_gemm(X, K, W, R, N, K, d_bias, gelu, static_cast<sw::bf16*>(d_out), N, d_partial, split, st,
-                         kernel == 1 ? -1 : 0);
+  if (kernel == 1) {
+    if (split <= 0) split = sw::skinny_mma_split_for(N, K);
+    return sw::skinny_gemm_mma(X, K, W, R, N, K, d_bias, gelu, static_cast<sw::bf16*>(d_out), N, d_partial, split, st);
+  }
+  if (split <= 0) split = sw::skinny_split_for(N, K);
+  return sw::skinny_gemm(X, K, W, R, N, K, d_bias, gelu, static_cast<sw::bf16*>(d_out), N, d_partial, split, st);
 }
 int sw_dev_skinny_split_k(int kernel, int N, int K) {
   return kernel == 2 ? sw::skinny_tc_split_for(N, K) : kernel == 1 ? sw::skinny_mma_split_for(N, K) : sw::skinny_split_for(N, K);

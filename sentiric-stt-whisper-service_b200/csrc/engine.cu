@@ -37,11 +37,6 @@ Engine::~Engine() {
   if (ev1) cudaEventDestroy(ev1);
   for (auto ev : xa_ev)
     if (ev) cudaEventDestroy(ev);
-  for (auto ev : ev_half)
-    if (ev) cudaEventDestroy(ev);
-  if (ev_fork) cudaEventDestroy(ev_fork);
-  if (ev_join) cudaEventDestroy(ev_join);
-  if (stream2) cudaStreamDestroy(stream2);
   engine_free_step_graphs(this);
   if (stream) cudaStreamDestroy(stream);
   if (post_stream) cudaStreamDestroy(post_stream);
@@ -66,12 +61,8 @@ static int engine_init(Engine* e, const char* path, const sw_ctx_params* p, cons
   SW_CHECK(e->max_beams <= 8, "max_beams %d > 8", e->max_beams);
   e->max_rows = std::max(8, e->max_batch * e->max_beams);  // any single window may run 8 decoders
   {
-    const char* a = getenv("SW_ATTN");  // development switch: SW_ATTN=legacy selects the mma.sync kernel
-    e->legacy_attention = a && strcmp(a, "legacy") == 0;
     const char* g = getenv("SW_GRAPHS");  // development switch: SW_GRAPHS=0 launches the step kernel by kernel
     e->use_graphs = !(g && strcmp(g, "0") == 0);
-    e->interleave = p && p->reserved[0] == 1;  // set by sw_ctx_create (lane mode "interleaved")
-    if (const char* mg = getenv("SW_INTERLEAVE_MIN")) e->interleave_min_groups = std::max(1, atoi(mg));  // tests: 1
   }
   size_t free0 = 0, total0 = 0;
   if (primary) {
@@ -84,11 +75,6 @@ static int engine_init(Engine* e, const char* path, const sw_ctx_params* p, cons
   cudaMemGetInfo(&free0, &total0);
   SW_CUDA_CHECK(cudaStreamCreateWithFlags(&e->stream, cudaStreamNonBlocking));
   SW_CUDA_CHECK(cudaStreamCreateWithFlags(&e->post_stream, cudaStreamNonBlocking));
-  SW_CUDA_CHECK(cudaStreamCreateWithFlags(&e->stream2, cudaStreamNonBlocking));
-  SW_CUDA_CHECK(cudaEventCreateWithFlags(&e->ev_fork, cudaEventDisableTiming));
-  SW_CUDA_CHECK(cudaEventCreateWithFlags(&e->ev_join, cudaEventDisableTiming));
-  e->ev_half.assign(2 * (size_t)64, nullptr);
-  for (auto& ev : e->ev_half) SW_CUDA_CHECK(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
   SW_CUDA_CHECK(cudaEventCreate(&e->ev0));
   SW_CUDA_CHECK(cudaEventCreate(&e->ev1));
   e->xa_ev.assign(2 * (size_t)64, nullptr);
@@ -109,7 +95,7 @@ static int engine_init(Engine* e, const char* path, const sw_ctx_params* p, cons
   e->logits_ld = (hp.n_vocab + 3) / 4 * 4;
   if (e->dx.alloc(R * d) || e->dh.alloc(R * d) || e->dqkv.alloc(R * 3 * d) || e->datt.alloc(R * d) ||
       e->dq.alloc(R * d) || e->dff.alloc(R * 4 * d) || e->logits.alloc(R * e->logits_ld) ||
-      e->xa_ws.alloc(2 * cross_attention_ws_floats((int)R, (int)d, hp.n_text_head)) || e->dpart.alloc(32 * R * d))
+      e->xa_ws.alloc(cross_attention_ws_floats((int)R, (int)d, hp.n_text_head)) || e->dpart.alloc(32 * R * d))
     return -1;
   e->n_pages = (int)(R * KV_MAX_PAGES + R);
   const size_t page_elems = (size_t)hp.n_text_layer * 2 * KV_PAGE * d;
@@ -158,23 +144,9 @@ Engine* engine_create_lane(const Engine* primary) {
   return e;
 }
 
-// development: SW_XA_TRACE=1 brackets EVERY layer's cross attention and prints, for three steps, each launch's start
-// and end on a process-wide time axis (stderr) - the phase relation of the lanes' cache streams
-static bool xa_trace() {
-  static const bool on = getenv("SW_XA_TRACE") && atoi(getenv("SW_XA_TRACE")) != 0;
-  return on;
-}
-static const int XA_TIMED_EVERY = xa_trace() ? 1 : (getenv("SW_XA_TIMED_EVERY") ? std::max(1, atoi(getenv("SW_XA_TIMED_EVERY"))) : 8);
-static cudaEvent_t xa_trace_origin() {
-  static cudaEvent_t ev = [] {
-    cudaEvent_t e = nullptr;
-    cudaEventCreate(&e);
-    cudaEventRecord(e, 0);
-    cudaEventSynchronize(e);
-    return e;
-  }();
-  return ev;
-}
+// kernel timing (bench roofline) brackets the cross attention of every 8th layer only: an event node between two
+// kernels turns their programmatic edge into a full dependency
+static constexpr int XA_TIMED_EVERY = 8;
 
 #define GEMM(args)                                   \
   do {                                               \
@@ -220,9 +192,7 @@ int engine_encode(Engine* e, int n_win, float* enc_out_f32) {
       a.bias = w.bqkv; a.M = (int)M; a.N = 3 * d; a.K = d;
       GEMM(a);
     }
-    if (e->legacy_attention ? encoder_attention(e->qkv.p, e->hb.p, n_win, 1500, d, hp.n_audio_head, st)
-                            : encoder_attention_tc(e->qkv.p, e->hb.p, n_win, 1500, d, hp.n_audio_head, st))
-      return -1;
+    if (encoder_attention_tc(e->qkv.p, e->hb.p, n_win, 1500, d, hp.n_audio_head, st)) return -1;
     {
       GemmArgs a;
       a.A = e->hb.p; a.lda = d; a.B = w.wo; a.ldb = d; a.C = e->x.p; a.ldc = d;
@@ -282,24 +252,8 @@ int engine_copy_pages(Engine* e, const std::vector<int>& pairs) {
 
 // Everything one decoder step puts on the stream (uploads, kernels, pick read-back). `launches`
 // counts kernels; `capturing` selects graph-safe event records for the kernel-timing probes.
-//
-// Interleaved halves (Engine::interleave, `split`): the windows of the step are cut into two halves that run
-// the layer stack as two dependency chains on two streams of the same graph. A decoder layer is a chain of
-// latency-bound kernels (58 us, almost no HBM traffic) followed by the cross attention that streams the layer's
-// cross-KV (85 us for 64 windows at 0.89 of HBM). Two independent lanes that start together stay in phase -
-// both stream, then both run their chains with HBM idle (228 us per layer pair, which is what was measured:
-// 0.72 of HBM). Here half B's chain is ordered to run under half A's cross attention and vice versa
-// (xattn A(l) -> xattn B(l) -> xattn A(l+1) as explicit edges), so the cache stream never pauses. The chain
-// kernels share SMs with the resident cross-attention CTAs (4-stage skinny ring: 53 KB next to 165 KB).
-struct StepHalf {
-  int r0, R;             // rows [r0, r0 + R) of the step
-  int g0, G, max_count;  // their windows (groups) and the largest group
-  float* part;           // split-K partial sums of this half: [split][R][d]
-  cudaStream_t st;
-};
-
 static int enqueue_decode_step(Engine* e, int R, int n_groups, int max_count, bool want_logits, int n_lrows,
-                               const LogitCfg& cfg, bool upload_page_table, bool capturing, bool split, long* launches) {
+                               const LogitCfg& cfg, bool upload_page_table, bool capturing, long* launches) {
   const Model& m = *e->model;
   const HParams& hp = m.hp;
   const int d = hp.n_text_state, L = hp.n_text_layer;
@@ -319,29 +273,13 @@ static int enqueue_decode_step(Engine* e, int R, int n_groups, int max_count, bo
   // cross-attention query are split along K; their f32 partial sums are folded in by the consumer
   // (the fused LayerNorm adds bias + partials into x; cross_attention reduces its query on load).
   const int sp_d = skinny_split_for(d, d), sp_ff = skinny_split_for(d, 4 * d);
-  // ---- the halves
-  StepHalf hv[2];
-  int n_half = 1;
-  hv[0] = StepHalf{0, R, 0, n_groups, max_count, e->dpart.p, st};
-  if (split) {
-    const int* g_start = e->h_grp.p + e->max_rows;
-    const int* g_count = e->h_grp.p + 2 * e->max_rows;
-    const int gA = n_groups / 2, rA = g_start[gA];
-    int mcA = 1, mcB = 1;
-    for (int g = 0; g < n_groups; ++g) (g < gA ? mcA : mcB) = std::max(g < gA ? mcA : mcB, g_count[g]);
-    hv[0] = StepHalf{0, rA, 0, gA, mcA, e->dpart.p, st};
-    hv[1] = StepHalf{rA, R - rA, gA, n_groups - gA, mcB, e->dpart.p + (size_t)32 * rA * d, e->stream2};
-    n_half = 2;
-    SW_CUDA_CHECK(cudaEventRecord(e->ev_fork, st));   // half B joins the capture behind the uploads and the embedding
-    SW_CUDA_CHECK(cudaStreamWaitEvent(e->stream2, e->ev_fork, 0));
-  }
-  const int sk_stages = split ? 4 : 0;  // co-resident with the other half's cross attention
+  const int64_t ps = (int64_t)R * d;  // stride between the K slices of the partial sums
+  float* part = e->dpart.p;
   const float* pend_bias = nullptr;  // bias of the FC2 partials still to be folded into x
   int pend_split = 0;
   // development switch: SW_SKIP=<bitmask> leaves kernels out of the step (results are garbage) so that
   // the in-graph cost of each one can be read off as a time difference (tools/dev_step_time.py)
   static const int skip = getenv("SW_SKIP") ? atoi(getenv("SW_SKIP")) : 0;
-  static const bool order_xattn = !(getenv("SW_INTERLEAVE_ORDER") && atoi(getenv("SW_INTERLEAVE_ORDER")) == 0);
 #define STEP_K(bit, call)                    \
   do {                                       \
     if (!(skip & (bit))) {                   \
@@ -351,74 +289,43 @@ static int enqueue_decode_step(Engine* e, int R, int n_groups, int max_count, bo
   } while (0)
   for (int l = 0; l < L; ++l) {
     const DecLayerW& w = m.dec[l];
-    for (int hi = 0; hi < n_half; ++hi) {
-      const StepHalf& h = hv[hi];
-      cudaStream_t hs = h.st;
-      const int64_t ps = (int64_t)h.R * d;  // stride between this half's K slices
-      float* x = e->dx.p + (int64_t)h.r0 * d;
-      bf16* hb = e->dh.p + (int64_t)h.r0 * d;
-      bf16* qkv = e->dqkv.p + (int64_t)h.r0 * 3 * d;
-      bf16* att = e->datt.p + (int64_t)h.r0 * d;
-      bf16* ff = e->dff.p + (int64_t)h.r0 * 4 * d;
-      STEP_K(1, layer_norm(x, h.R, d, w.ln1.g, w.ln1.b, hb, nullptr, pend_split ? h.part : nullptr, pend_split, ps,
-                           pend_bias, hs));
-      STEP_K(2, skinny_gemm(hb, d, w.wqkv, h.R, 3 * d, d, w.bqkv, 0, qkv, 3 * d, nullptr, 1, hs, sk_stages));
-      STEP_K(4, self_attention(qkv, e->d_rows.p + h.r0, h.R, d, hp.n_text_head, e->kv_pool.p, l, L, att, hs));
-      STEP_K(8, skinny_gemm(att, d, w.wo, h.R, d, d, nullptr, 0, nullptr, 0, h.part, sp_d, hs, sk_stages));
-      STEP_K(1, layer_norm(x, h.R, d, w.lnx.g, w.lnx.b, hb, nullptr, h.part, sp_d, ps, w.bo, hs));
-      STEP_K(16, skinny_gemm(hb, d, w.wxq, h.R, d, d, nullptr, 0, nullptr, 0, h.part, sp_d, hs, sk_stages));
-      STEP_K(32, reduce_partials(h.part, sp_d, ps, h.R, d, w.bxq, e->dq.p + (int64_t)h.r0 * d, hs));
-      // kernel-timing probes bracket the cross attention of every XA_TIMED_EVERY-th layer only (first half): an
-      // event node between two kernels turns their programmatic edge into a full dependency
-      const bool timed = e->kernel_timing && hi == 0 && l % XA_TIMED_EVERY == 0;
-      if (timed) SW_CUDA_CHECK(cudaEventRecordWithFlags(e->xa_ev[2 * l], hs, ev_flags));
-      if (!(skip & 64)) {
-        // the cache stream alternates between the halves: A(l) -> B(l) -> A(l+1) ...
-        cudaEvent_t ev_dep = nullptr;
-        if (split && order_xattn) {
-          if (hi == 0 && l > 0) SW_CUDA_CHECK(cudaStreamWaitEvent(hs, e->ev_half[2 * (l - 1) + 1], 0));
-          if (hi == 1) SW_CUDA_CHECK(cudaStreamWaitEvent(hs, e->ev_half[2 * l], 0));
-          ev_dep = e->ev_half[2 * l + hi];
-        }
-        // q / out are addressed by absolute rows (grp_start); each half has its own half of the partials buffer
-        float* ws = e->xa_ws.p + (hi ? e->xa_ws.n / 2 : 0);
-        if (cross_attention(e->dq.p, e->cross_kv.p + l * layer_stride, (int64_t)e->max_batch * 1500,
-                            e->d_grp_win.p + h.g0, e->d_grp_start.p + h.g0, e->d_grp_count.p + h.g0, h.G, h.max_count, h.R,
-                            1500, d, hp.n_text_head, ws, e->datt.p, hs, timed ? e->xa_ev[2 * l + 1] : nullptr, ev_flags,
-                            e->xa_max_ctas, h.r0, ev_dep))
-          return -1;
-        *launches += 2;
-      } else if (timed) {
-        SW_CUDA_CHECK(cudaEventRecordWithFlags(e->xa_ev[2 * l + 1], hs, ev_flags));
-      }
-      STEP_K(256, skinny_gemm(att, d, w.wxo, h.R, d, d, nullptr, 0, nullptr, 0, h.part, sp_d, hs, sk_stages));
-      STEP_K(1, layer_norm(x, h.R, d, w.ln2.g, w.ln2.b, hb, nullptr, h.part, sp_d, ps, w.bxo, hs));
-      STEP_K(512, skinny_gemm(hb, d, w.w1, h.R, 4 * d, d, w.b1, 1, ff, 4 * d, nullptr, 1, hs, sk_stages));
-      STEP_K(1024, skinny_gemm(ff, 4 * d, w.w2, h.R, d, 4 * d, nullptr, 0, nullptr, 0, h.part, sp_ff, hs, sk_stages));
+    STEP_K(1, layer_norm(e->dx.p, R, d, w.ln1.g, w.ln1.b, e->dh.p, nullptr, pend_split ? part : nullptr, pend_split, ps,
+                         pend_bias, st));
+    STEP_K(2, skinny_gemm(e->dh.p, d, w.wqkv, R, 3 * d, d, w.bqkv, 0, e->dqkv.p, 3 * d, nullptr, 1, st));
+    STEP_K(4, self_attention(e->dqkv.p, e->d_rows.p, R, d, hp.n_text_head, e->kv_pool.p, l, L, e->datt.p, st));
+    STEP_K(8, skinny_gemm(e->datt.p, d, w.wo, R, d, d, nullptr, 0, nullptr, 0, part, sp_d, st));
+    STEP_K(1, layer_norm(e->dx.p, R, d, w.lnx.g, w.lnx.b, e->dh.p, nullptr, part, sp_d, ps, w.bo, st));
+    STEP_K(16, skinny_gemm(e->dh.p, d, w.wxq, R, d, d, nullptr, 0, nullptr, 0, part, sp_d, st));
+    STEP_K(32, reduce_partials(part, sp_d, ps, R, d, w.bxq, e->dq.p, st));
+    const bool timed = e->kernel_timing && l % XA_TIMED_EVERY == 0;
+    if (timed) SW_CUDA_CHECK(cudaEventRecordWithFlags(e->xa_ev[2 * l], st, ev_flags));
+    if (!(skip & 64)) {
+      if (cross_attention(e->dq.p, e->cross_kv.p + l * layer_stride, (int64_t)e->max_batch * 1500, e->d_grp_win.p,
+                          e->d_grp_start.p, e->d_grp_count.p, n_groups, max_count, R, 1500, d, hp.n_text_head,
+                          e->xa_ws.p, e->datt.p, st, timed ? e->xa_ev[2 * l + 1] : nullptr, ev_flags, e->xa_max_ctas))
+        return -1;
+      *launches += 2;
+    } else if (timed) {
+      SW_CUDA_CHECK(cudaEventRecordWithFlags(e->xa_ev[2 * l + 1], st, ev_flags));
     }
+    STEP_K(256, skinny_gemm(e->datt.p, d, w.wxo, R, d, d, nullptr, 0, nullptr, 0, part, sp_d, st));
+    STEP_K(1, layer_norm(e->dx.p, R, d, w.ln2.g, w.ln2.b, e->dh.p, nullptr, part, sp_d, ps, w.bxo, st));
+    STEP_K(512, skinny_gemm(e->dh.p, d, w.w1, R, 4 * d, d, w.b1, 1, e->dff.p, 4 * d, nullptr, 1, st));
+    STEP_K(1024, skinny_gemm(e->dff.p, 4 * d, w.w2, R, d, 4 * d, nullptr, 0, nullptr, 0, part, sp_ff, st));
     pend_bias = w.b2;
     pend_split = sp_ff;
   }
 #undef STEP_K
   (*launches) += 1;
-  if (want_logits || n_lrows > 0) {
-    for (int hi = 0; hi < n_half; ++hi) {  // the final LayerNorm folds each half's last FC2 partials in
-      const StepHalf& h = hv[hi];
-      if (layer_norm(e->dx.p + (int64_t)h.r0 * d, h.R, d, m.dec_ln.g, m.dec_ln.b, e->dh.p + (int64_t)h.r0 * d, nullptr,
-                     pend_split ? h.part : nullptr, pend_split, (int64_t)h.R * d, pend_bias, h.st))
-        return -1;
-      (*launches) += 1;
-    }
-  }
-  if (split) {  // join: everything below runs behind both halves
-    SW_CUDA_CHECK(cudaEventRecord(e->ev_join, e->stream2));
-    SW_CUDA_CHECK(cudaStreamWaitEvent(st, e->ev_join, 0));
-  }
-  if (want_logits || n_lrows > 0) {
+  if (want_logits || n_lrows > 0) {  // the final LayerNorm folds the last FC2 partials in
+    if (layer_norm(e->dx.p, R, d, m.dec_ln.g, m.dec_ln.b, e->dh.p, nullptr, pend_split ? part : nullptr, pend_split,
+                   ps, pend_bias, st))
+      return -1;
+    (*launches) += 1;
     GemmArgs a;
     a.A = e->dh.p; a.lda = d; a.B = m.tok_emb; a.ldb = d; a.C = e->logits.p; a.ldc = e->logits_ld;
     a.M = R; a.N = hp.n_vocab; a.K = d; a.flags = GEMM_OUT_F32;
-    if (gemm_bf16_tn(a, e->stream)) return -1;
+    if (gemm_bf16_tn(a, st)) return -1;
     (*launches) += 1;
   }
   if (n_lrows > 0) {
@@ -436,12 +343,10 @@ static int enqueue_decode_step(Engine* e, int R, int n_groups, int max_count, bo
 // their contents are refreshed per run / per step.
 struct StepKey {
   int R, G, max_count, want_logits, n_lrows, upload_pt, timing, suppress_blank, max_initial_ts_id;
-  int split_row, max_count_b;  // interleaved halves: where the rows are cut and half B's largest group (0: one chain)
   bool operator<(const StepKey& o) const {
-    return std::tie(R, G, max_count, want_logits, n_lrows, upload_pt, timing, suppress_blank, max_initial_ts_id,
-                    split_row, max_count_b) <
+    return std::tie(R, G, max_count, want_logits, n_lrows, upload_pt, timing, suppress_blank, max_initial_ts_id) <
            std::tie(o.R, o.G, o.max_count, o.want_logits, o.n_lrows, o.upload_pt, o.timing, o.suppress_blank,
-                    o.max_initial_ts_id, o.split_row, o.max_count_b);
+                    o.max_initial_ts_id);
   }
 };
 struct StepGraph {
@@ -470,22 +375,10 @@ int engine_decode_step(Engine* e, int R, int n_groups, int max_count, bool want_
   for (int r = 0; r < R; ++r)  // each row carries its slot's page list (the host table is the pager's)
     memcpy(e->h_rows.p[r].pages, e->h_page_table.p + (size_t)e->h_rows.p[r].slot * KV_MAX_PAGES,
            KV_MAX_PAGES * sizeof(int));
-  // interleaved halves: worth it when both halves carry enough windows to stream for longer than a chain lasts
-  const bool split = e->interleave && n_groups >= 2 * e->interleave_min_groups;
-  int split_row = 0, mc_a = max_count, mc_b = 0;
-  if (split) {
-    const int* g_start = e->h_grp.p + e->max_rows;
-    const int* g_count = e->h_grp.p + 2 * e->max_rows;
-    split_row = g_start[n_groups / 2];
-    mc_a = 1;
-    mc_b = 1;
-    for (int g = 0; g < n_groups; ++g) (g < n_groups / 2 ? mc_a : mc_b) = std::max(g < n_groups / 2 ? mc_a : mc_b, g_count[g]);
-  }
   if (!e->use_graphs) {
     SW_CUDA_CHECK(cudaEventRecord(e->ev0, st));
     long launches = 0;
-    if (enqueue_decode_step(e, R, n_groups, max_count, want_logits, n_lrows, cfg, upload_page_table, false, split,
-                            &launches))
+    if (enqueue_decode_step(e, R, n_groups, max_count, want_logits, n_lrows, cfg, upload_page_table, false, &launches))
       return -1;
     e->times.n_launches += launches;
   } else {
@@ -493,8 +386,8 @@ int engine_decode_step(Engine* e, int R, int n_groups, int max_count, bool want_
     // it (one host call per step instead of ~460, and no inter-kernel launch gaps).
     if (!e->step_graphs) e->step_graphs = new StepGraphCache();
     StepGraphCache& cache = *static_cast<StepGraphCache*>(e->step_graphs);
-    const StepKey key{R, n_groups, split ? mc_a : max_count, want_logits ? 1 : 0, n_lrows, 0, e->kernel_timing ? 1 : 0,
-                      cfg.suppress_blank, cfg.max_initial_ts_id, split_row, mc_b};
+    const StepKey key{R, n_groups, max_count, want_logits ? 1 : 0, n_lrows, 0, e->kernel_timing ? 1 : 0,
+                      cfg.suppress_blank, cfg.max_initial_ts_id};
     auto it = cache.graphs.find(key);
     if (it == cache.graphs.end()) {
       if (cache.graphs.size() > 512) {  // bounded: drop everything and start over
@@ -504,7 +397,7 @@ int engine_decode_step(Engine* e, int R, int n_groups, int max_count, bool want_
       StepGraph g;
       SW_CUDA_CHECK(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
       const int rc = enqueue_decode_step(e, R, n_groups, max_count, want_logits, n_lrows, cfg, upload_page_table,
-                                         true, split, &g.launches);
+                                         true, &g.launches);
       cudaGraph_t graph = nullptr;
       const cudaError_t ce = cudaStreamEndCapture(st, &graph);
       if (rc || ce != cudaSuccess || !graph) {
@@ -537,18 +430,6 @@ int engine_decode_step(Engine* e, int R, int n_groups, int max_count, bool want_
       e->times.ms_xattn += t;
     }
     e->times.n_xattn += n_timed;
-    if (xa_trace() && e->times.n_steps >= 40 && e->times.n_steps < 43) {
-      float s0 = 0, s1 = 0;
-      cudaEventElapsedTime(&s0, xa_trace_origin(), e->ev0);
-      cudaEventElapsedTime(&s1, xa_trace_origin(), e->ev1);
-      fprintf(stderr, "XATRACE eng %p step %ld begin %.1f end %.1f us\n", (void*)e, e->times.n_steps, s0 * 1e3, s1 * 1e3);
-      for (int l = 0; l < L; ++l) {
-        float t0 = 0, t1 = 0;
-        cudaEventElapsedTime(&t0, xa_trace_origin(), e->xa_ev[2 * l]);
-        cudaEventElapsedTime(&t1, xa_trace_origin(), e->xa_ev[2 * l + 1]);
-        fprintf(stderr, "XATRACE eng %p step %ld layer %d xattn %.1f .. %.1f us\n", (void*)e, e->times.n_steps, l, t0 * 1e3, t1 * 1e3);
-      }
-    }
     // per launch: the cross-KV of every active window once + q in + attention out
     e->times.xattn_bytes += (double)n_timed * ((double)n_groups * 1500 * 2 * d * 2 + (double)R * d * 4);
   }

@@ -84,13 +84,6 @@ struct Engine {
   // token-time refinement of a finished batch (token_times.cu), on its own stream: it runs from the host
   // thread that post-processes batch i while the main stream already decodes batch i + 1
   cudaStream_t post_stream = nullptr;
-  // interleaved halves of a decoder step (engine.cu::enqueue_decode_step): second stream of the step graph and
-  // the events that order the two halves' cross attentions
-  bool interleave = false;
-  int interleave_min_groups = 8;  // per half
-  cudaStream_t stream2 = nullptr;
-  cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
-  std::vector<cudaEvent_t> ev_half;
   DevBuf<TtSeg> d_tt_seg;
   PinBuf<TtSeg> h_tt_seg;
   DevBuf<long long> d_tt_t;     // t0 | t1 (two halves of tt_tok_capacity)
@@ -123,7 +116,6 @@ struct Engine {
 
   StageTimes times;
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
-  bool legacy_attention = false;
   bool use_graphs = true;       // replay each decoder step from a CUDA graph captured per step shape
   void* step_graphs = nullptr;  // StepGraphCache (engine.cu)
   bool kernel_timing = false;   // bracket each cross_attention launch with events (bench roofline)

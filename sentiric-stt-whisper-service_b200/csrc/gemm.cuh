@@ -33,7 +33,8 @@ struct GemmArgs {
   int res_mod = 0;  // >0: residual row = m % res_mod
   int M = 0, N = 0, K = 0, batch = 1;
   int flags = 0;
-  int block_n = 0;  // 0 = auto (64/128/256)
+  int block_n = 0;  // 0 = auto (64/128/256, or CTA pairs for M >= 2048 at 256); 64/128/256: that single-CTA tile;
+                    // 512: CTA pairs (2 x 256)
 };
 
 // Enqueue on `stream`. Returns 0 or -1 (see sw_last_error()).

@@ -610,10 +610,8 @@ int make_operand_map(CUtensorMap* map, const void* base, int64_t K, int64_t rows
 }
 
 // 256-bit epilogue accesses need 32-byte aligned rows of C (and of the residual, when there is one);
-// development switch: SW_GEMM_NARROW=1 keeps the 128-bit accesses
+// otherwise the epilogue keeps 128-bit accesses
 bool epilogue_wide_ok(const GemmArgs& a) {
-  static const bool narrow = getenv("SW_GEMM_NARROW") != nullptr;
-  if (narrow) return false;
   const int64_t esz = (a.flags & GEMM_OUT_F32) ? 4 : 2;
   bool ok = (reinterpret_cast<uintptr_t>(a.C) & 31) == 0 && (a.ldc * esz) % 32 == 0 && (a.c_batch_stride * esz) % 32 == 0;
   if (a.residual)
@@ -731,13 +729,9 @@ int gemm_bf16_tn(const GemmArgs& a, cudaStream_t stream) {
     bn = 256;
     while (bn > 64 && (m_tiles * ((a.N + bn - 1) / bn) * a.batch < num_sms() || a.N <= bn / 2))
       bn >>= 1;
+    if (bn == 256 && a.M >= 2048) bn = 512;  // CTA pairs for the large encoder shapes
   }
-  // CTA pairs for the large encoder shapes (development switch: SW_GEMM_PAIR=0/1, block_n = 512 forces it)
-  static const int pair_on = [] {
-    const char* e = getenv("SW_GEMM_PAIR");
-    return e ? atoi(e) : 1;
-  }();
-  if (bn == 512 || (pair_on && bn == 256 && a.M >= 2048)) return launch_pair(a, stream);
+  if (bn == 512) return launch_pair(a, stream);
   switch (bn) {
     case 64: return launch<64>(a, stream);
     case 128: return launch<128>(a, stream);

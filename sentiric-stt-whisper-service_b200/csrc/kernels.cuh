@@ -80,11 +80,9 @@ int embed_tokens(const bf16* tok_emb, const float* pos_emb, const int* d_tok, co
 int convert_f16_to_bf16(const uint16_t* src, bf16* dst, int64_t n, cudaStream_t stream);
 int convert_f32_to_bf16(const float* src, bf16* dst, int64_t n, cudaStream_t stream);
 
-// ------------------------------------------------------------------ encoder attention (attn_enc.cu)
+// ------------------------------------------------------------------ encoder attention (attn_enc_tc.cu)
 // non-causal MHA over T keys per (window, head); qkv [n_win*T][3d] bf16 (Q | K | V), out [n_win*T][d].
-int encoder_attention(const bf16* qkv, bf16* out, int n_win, int T, int d, int n_head,
-                      cudaStream_t stream);
-// generation 2: tcgen05 / TMEM / TMA flash attention (attn_enc_tc.cu); same contract
+// tcgen05 / TMEM / TMA flash attention
 int encoder_attention_tc(const bf16* qkv, bf16* out, int n_win, int T, int d, int n_head,
                          cudaStream_t stream);
 
@@ -121,17 +119,16 @@ int cross_attention(const bf16* q, const bf16* kv, int64_t kv_rows, const int* d
                     const int* d_grp_start, const int* d_grp_count, int n_groups, int max_count, int R,
                     int T, int d, int n_head, float* ws, bf16* out, cudaStream_t stream,
                     cudaEvent_t ev_main_done = nullptr, unsigned ev_flags = 0,  // event after the main kernel
-                    int max_ctas = 0,   // cap on the persistent grid (0 = one CTA per SM)
-                    int row0 = 0,       // the groups cover rows [row0, row0 + R) of q / ws / out (grp_start is absolute)
-                    cudaEvent_t ev_dep = nullptr);  // plain record after the main kernel (a dependency edge for another stream)
+                    int max_ctas = 0);  // cap on the persistent grid (0 = one CTA per SM)
 
 // weight-streaming GEMM for <= 64-row blocks (skinny_gemm.cu): out = X . W^T
 //   split == 1: out bf16 [R][ldo] = act(acc + bias);   split > 1: partial f32 [split][R][N] (raw sums)
 int skinny_split_for(int N, int K);
-// stages: depth of the shared-memory ring (0 = default 8; 4 = 53 KB per CTA, small enough to share an SM with a
-// resident cross-attention CTA)
 int skinny_gemm(const bf16* X, int ldx, const bf16* W, int R, int N, int K, const float* bias, int gelu,
-                bf16* out, int ldo, float* partial, int split, cudaStream_t stream, int stages = 0);
+                bf16* out, int ldo, float* partial, int split, cudaStream_t stream);
+// the mma.sync kernel whatever skinny_use_tc says (skinny_gemm() routes the shapes skinny_use_tc rejects here)
+int skinny_gemm_mma(const bf16* X, int ldx, const bf16* W, int R, int N, int K, const float* bias, int gelu,
+                    bf16* out, int ldo, float* partial, int split, cudaStream_t stream);
 // generation 3 (skinny_gemm_tc.cu): 128 weight rows per CTA in the M dimension of tcgen05.mma; skinny_gemm() and
 // skinny_split_for() route the wide models' matrices to it (skinny_use_tc)
 bool skinny_use_tc(int N, int K);

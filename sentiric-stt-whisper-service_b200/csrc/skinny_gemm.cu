@@ -221,42 +221,36 @@ int skinny_mma_split_for(int N, int K) {
 }
 
 int skinny_gemm(const bf16* X, int ldx, const bf16* W, int R, int N, int K, const float* bias, int gelu,
-                bf16* out, int ldo, float* partial, int split, cudaStream_t stream, int stages) {
+                bf16* out, int ldo, float* partial, int split, cudaStream_t stream) {
+  if (skinny_use_tc(N, K)) return skinny_gemm_tc(X, ldx, W, R, N, K, bias, gelu, out, ldo, partial, split, stream);
+  return skinny_gemm_mma(X, ldx, W, R, N, K, bias, gelu, out, ldo, partial, split, stream);
+}
+
+int skinny_gemm_mma(const bf16* X, int ldx, const bf16* W, int R, int N, int K, const float* bias, int gelu,
+                    bf16* out, int ldo, float* partial, int split, cudaStream_t stream) {
   if (R <= 0) return 0;
-  if (stages >= 0 && skinny_use_tc(N, K))  // stages < 0: this kernel whatever the shape (development hook)
-    return skinny_gemm_tc(X, ldx, W, R, N, K, bias, gelu, out, ldo, partial, split, stream);
   SW_CHECK(K % SK_BK == 0 && ldx % 8 == 0 && N % 2 == 0, "skinny_gemm: unsupported shape N=%d K=%d ldx=%d", N, K, ldx);
   SW_CHECK(split >= 1 && split <= 32 && (split == 1 || partial), "skinny_gemm: split-K needs a partial buffer");
   SW_CHECK(K % (split * SK_BK) == 0, "skinny_gemm: K=%d not divisible into %d slices of 64-element blocks", K, split);
   SW_CHECK(partial || out, "skinny_gemm: null output");
   SW_CHECK((reinterpret_cast<uintptr_t>(X) & 15) == 0 && (reinterpret_cast<uintptr_t>(W) & 15) == 0,
            "skinny_gemm: operands must be 16-byte aligned");
-  // ring depth: 8 stages (two CTAs of ~100 KB per SM) when the launch has the GPU to itself; SW_SKINNY_STAGES
-  // selects a shallower ring (development: 4 stages = 53 KB, small enough to share an SM with a resident
-  // cross-attention CTA of the other lane)
-  static const int env_stages = [] {
-    const char* v = getenv("SW_SKINNY_STAGES");
-    const int n = v ? atoi(v) : 0;
-    return n >= 2 && n <= SK_STAGES ? n : 0;
-  }();
-  const int n_stages = env_stages ? env_stages : (stages >= 2 && stages <= SK_STAGES ? stages : SK_STAGES);
   static SmemOptIn opt_in32, opt_in40;  // per device (host_common.h)
   SW_CUDA_CHECK(opt_in32.ensure(skinny_gemm_kernel<32>, SkCfg<32>::smem(SK_STAGES)));
   SW_CUDA_CHECK(opt_in40.ensure(skinny_gemm_kernel<40>, SkCfg<40>::smem(SK_STAGES)));
   const int k_slice = K / split;
   const int row_blocks = (R + SK_BM - 1) / SK_BM;
-  static const int force_bn = getenv("SW_SKINNY_BN") ? atoi(getenv("SW_SKINNY_BN")) : 0;  // development switch
-  const int bn = force_bn ? force_bn : sk_pick_bn(N, K, row_blocks, split);
+  const int bn = sk_pick_bn(N, K, row_blocks, split);
   CUtensorMap map_x, map_w;
   if (make_tma_map_2d_bf16(&map_x, X, K, R, ldx, SK_BK, SK_BM)) return -1;
   if (make_tma_map_2d_bf16(&map_w, W, K, N, K, SK_BK, bn)) return -1;
   dim3 grid((N + bn - 1) / bn, split, row_blocks);
   if (bn == 40)
-    SW_CUDA_CHECK(launch_pdl(skinny_gemm_kernel<40>, grid, dim3(SK_THREADS), SkCfg<40>::smem(n_stages), stream, map_x,
-                             map_w, R, N, k_slice, bias, gelu, out, ldo, partial, 0u, n_stages));
+    SW_CUDA_CHECK(launch_pdl(skinny_gemm_kernel<40>, grid, dim3(SK_THREADS), SkCfg<40>::smem(SK_STAGES), stream, map_x,
+                             map_w, R, N, k_slice, bias, gelu, out, ldo, partial, 0u, SK_STAGES));
   else
-    SW_CUDA_CHECK(launch_pdl(skinny_gemm_kernel<32>, grid, dim3(SK_THREADS), SkCfg<32>::smem(n_stages), stream, map_x,
-                             map_w, R, N, k_slice, bias, gelu, out, ldo, partial, 0u, n_stages));
+    SW_CUDA_CHECK(launch_pdl(skinny_gemm_kernel<32>, grid, dim3(SK_THREADS), SkCfg<32>::smem(SK_STAGES), stream, map_x,
+                             map_w, R, N, k_slice, bias, gelu, out, ldo, partial, 0u, SK_STAGES));
   return 0;
 }
 

@@ -16,8 +16,6 @@
 //                covers 32 consecutive outputs (128 B of f32 partials, 64 B of bf16)
 // The accumulator is the TRANSPOSE of the output tile; bias is per lane. Split-K partials are f32 [split][R][N]
 // exactly as in skinny_gemm.cu, so the consumers (fused LayerNorm, reduce_partials) do not change.
-#include <stdlib.h>
-
 #include "common.cuh"
 #include "gemm.cuh"
 #include "kernels.cuh"
@@ -33,7 +31,7 @@ constexpr int ST_MAX_STAGES = 8;
 __global__ void __launch_bounds__(ST_THREADS, 1)
 skinny_gemm_tc_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_constant__ CUtensorMap map_x, int R, int N,
                       int k_slice, const float* __restrict__ bias, int gelu, bf16* __restrict__ out, int ldo,
-                      float* __restrict__ partial, int RB, int n_stages, int tmem_cols, int evict_last) {
+                      float* __restrict__ partial, int RB, int n_stages, int tmem_cols) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~static_cast<uintptr_t>(1023));
   const int stage_bytes = ST_W_BYTES + RB * ST_BK * 2;
@@ -71,11 +69,9 @@ skinny_gemm_tc_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_co
     if (elect_one_sync()) {
       // weights first (they do not depend on the predecessor), activations once it has finished
       const int pre = n_kb < n_stages ? n_kb : n_stages;
-      const uint64_t pol = l2_policy_evict_last();
       for (int kb = 0; kb < pre; ++kb) {
         mbar_arrive_expect_tx(&full[kb], stage_bytes);
-        if (evict_last) tma_load_2d_hint(smem + kb * stage_bytes, &map_w, &full[kb], k_begin + kb * ST_BK, n0, pol);
-        else tma_load_2d(smem + kb * stage_bytes, &map_w, &full[kb], k_begin + kb * ST_BK, n0);
+        tma_load_2d(smem + kb * stage_bytes, &map_w, &full[kb], k_begin + kb * ST_BK, n0);
       }
       pdl_wait();
       for (int kb = 0; kb < pre; ++kb)
@@ -85,8 +81,7 @@ skinny_gemm_tc_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_co
         mbar_wait(&empty[s], ((kb / n_stages) & 1) ^ 1);
         mbar_arrive_expect_tx(&full[s], stage_bytes);
         uint8_t* ws = smem + s * stage_bytes;
-        if (evict_last) tma_load_2d_hint(ws, &map_w, &full[s], k_begin + kb * ST_BK, n0, pol);
-        else tma_load_2d(ws, &map_w, &full[s], k_begin + kb * ST_BK, n0);
+        tma_load_2d(ws, &map_w, &full[s], k_begin + kb * ST_BK, n0);
         tma_load_2d(ws + ST_W_BYTES, &map_x, &full[s], k_begin + kb * ST_BK, r0);
       }
     }
@@ -145,18 +140,10 @@ skinny_gemm_tc_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_co
   }
 }
 
-// development switch: SW_SKINNY_TC=0 keeps every decoder GEMM on the mma.sync kernel, =2 forces this one for every
-// shape it supports
-int tc_mode() {
-  static const int m = getenv("SW_SKINNY_TC") ? atoi(getenv("SW_SKINNY_TC")) : 1;
-  return m;
-}
-
 }  // namespace
 
 bool skinny_use_tc(int N, int K) {
-  if (tc_mode() == 0 || K % ST_BK) return false;
-  if (tc_mode() == 2) return true;
+  if (K % ST_BK) return false;
   // small (d = 768) and wider: measured on BASELINE config 3 (small, beam 5) 9 654 -> 9 980 audio-s/s, config 2
   // (base, d = 512) unchanged - below that a matrix has too few 128-row tiles to stream from
   return N >= 768 && K >= 768;
@@ -197,11 +184,9 @@ int skinny_gemm_tc(const bf16* X, int ldx, const bf16* W, int R, int N, int K, c
   CUtensorMap map_w, map_x;
   if (make_tma_map_2d_bf16(&map_w, W, K, N, K, ST_BK, ST_BM)) return -1;
   if (make_tma_map_2d_bf16(&map_x, X, K, R, ldx, ST_BK, RB)) return -1;
-  // development switch: keep the weights in L2 for the other lane, which needs the same layer ~100 us later
-  static const int evict_last = getenv("SW_SKINNY_EVICT_LAST") ? atoi(getenv("SW_SKINNY_EVICT_LAST")) : 0;
   dim3 grid((N + ST_BM - 1) / ST_BM, split, row_blocks);
   SW_CUDA_CHECK(launch_pdl(skinny_gemm_tc_kernel, grid, dim3(ST_THREADS), smem, stream, map_w, map_x, R, N, k_slice, bias,
-                           gelu, out, ldo, partial, RB, n_stages, tmem_cols, evict_last));
+                           gelu, out, ldo, partial, RB, n_stages, tmem_cols));
   return 0;
 }
 

@@ -44,8 +44,7 @@ __global__ void __launch_bounds__((XA_MAX_CONSUMERS + 1) * 32, 1)
 cross_attention_kernel(const __grid_constant__ CUtensorMap map_kv, const bf16* __restrict__ q,
                        const int* __restrict__ grp_win, const int* __restrict__ grp_start,
                        const int* __restrict__ grp_count, int T, int d, int n_head, int n_cons, int spc,
-                       int n_stages, int n_chunks, int n_items, float* __restrict__ ws, uint32_t zero, int n_hsplit,
-                       int evict_first) {
+                       int n_stages, int n_chunks, int n_items, float* __restrict__ ws, uint32_t zero, int n_hsplit) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~static_cast<uintptr_t>(1023));
   const uint32_t sbase = smem_u32(smem);
@@ -77,6 +76,9 @@ cross_attention_kernel(const __grid_constant__ CUtensorMap map_kv, const bf16* _
     // no pdl_wait here: the cross-KV cache and the group tables were complete before the step's
     // first kernel started; the loads only fill this CTA's own shared memory
     if (elect_one_sync()) {  // not a lane test: one UTMALDG per load instead of a loop over the active lanes
+      // the cache is read once per step: evict-first keeps it from pushing the lanes' shared weights out of L2
+      // (+1.2 % on the two-lane bench against the default policy, measured ABAB on one box: 3 796 / 3 851 / 3 809 /
+      // 3 844 audio-s/s)
       const uint64_t pol = l2_policy_evict_first();
       int it = 0;
       for (int item = blockIdx.x; item < n_items; item += gridDim.x) {
@@ -93,14 +95,11 @@ cross_attention_kernel(const __grid_constant__ CUtensorMap map_kv, const bf16* _
           mbar_arrive_expect_tx(&full[s], stage_bytes);
           uint8_t* dst = smem + (size_t)s * stage_bytes;
           const int key = win * T + key_begin + i * XA_KEYS;
-          // segments of the [K row | V row] cache line: K heads 0 .. n_head-1, then V heads
-          if (evict_first) {  // the cache is read once per step: do not let it push the lanes' shared weights out of L2
-            tma_load_3d_hint(dst, &map_kv, &full[s], 0, key, hh * nh_cta, pol);
-            tma_load_3d_hint(dst + half_bytes, &map_kv, &full[s], 0, key, n_head + hh * nh_cta, pol);
-          } else {
-            tma_load_3d(dst, &map_kv, &full[s], 0, key, hh * nh_cta);
-            tma_load_3d(dst + half_bytes, &map_kv, &full[s], 0, key, n_head + hh * nh_cta);
-          }
+          // segments of the [K row | V row] cache line: K heads 0 .. n_head-1, then V heads. Not unrolled: with the
+          // two loads written out, ptxas spills more in the consumers of the 2- and 3-heads-per-warp instantiations
+#pragma unroll 1
+          for (int kv = 0; kv < 2; ++kv)
+            tma_load_3d_hint(dst + kv * half_bytes, &map_kv, &full[s], 0, key, kv * n_head + hh * nh_cta, pol);
         }
       }
     }
@@ -322,8 +321,6 @@ void xa_plan(int n_groups, int T, int d, int max_ctas, int n_hsplit, int* spc_ou
   int ns = (220 * 1024) / stage_bytes;
   if (ns > 8) ns = 8;
   if (ns < 2) ns = 2;
-  static const int env_ns = getenv("SW_XA_STAGES") ? atoi(getenv("SW_XA_STAGES")) : 0;  // development switch
-  if (env_ns >= 2 && env_ns < ns) ns = env_ns;
   *n_stages = ns;
 }
 
@@ -336,16 +333,15 @@ size_t cross_attention_ws_floats(int R, int d, int n_head) {
 int cross_attention(const bf16* q, const bf16* kv, int64_t kv_rows, const int* d_grp_win,
                     const int* d_grp_start, const int* d_grp_count, int n_groups, int max_count, int R,
                     int T, int d, int n_head, float* ws, bf16* out, cudaStream_t stream,
-                    cudaEvent_t ev_main_done, unsigned ev_flags, int max_ctas, int row0, cudaEvent_t ev_dep) {
+                    cudaEvent_t ev_main_done, unsigned ev_flags, int max_ctas) {
   if (n_groups <= 0 || R <= 0) return 0;
   SW_CHECK(d == n_head * 64, "cross_attention: head dim must be 64");
   SW_CHECK(max_count >= 1 && max_count <= 8, "cross_attention: group of %d rows", max_count);
   // wide models: a CTA takes half the heads of a (window, chunk), so a stage is 40 KB instead of 80 KB (large-v3) and
   // the ring 5 deep instead of 2 - with two stages an SM streamed 55 GB/s whatever the grid (64, 96 CTAs measured),
-  // i.e. the ring, not HBM, bounded every capped launch. SW_XA_HSPLIT=1 restores whole windows per CTA (development).
-  static const int force_hsplit = getenv("SW_XA_HSPLIT") ? atoi(getenv("SW_XA_HSPLIT")) : 0;
-  int n_hsplit = (XA_KEYS * 2 * d * 2 * 3 > 220 * 1024 && n_head % 2 == 0) ? 2 : 1;
-  if (force_hsplit == 1 || (force_hsplit == 2 && n_head % 2 == 0)) n_hsplit = force_hsplit;
+  // i.e. the ring, not HBM, bounded every capped launch. Narrow models, whose ring of whole-window stages is 3 or
+  // more deep, keep whole windows per CTA.
+  const int n_hsplit = (XA_KEYS * 2 * d * 2 * 3 > 220 * 1024 && n_head % 2 == 0) ? 2 : 1;
   const int nh_cta = n_head / n_hsplit;
   // consumer warps: the largest divisor of the item's heads that is <= 10, so every warp owns the same number of heads
   int n_cons = 1;
@@ -367,19 +363,13 @@ int cross_attention(const bf16* q, const bf16* kv, int64_t kv_rows, const int* d
   const int box[3] = {64, XA_KEYS, nh_cta};
   if (make_tma_map_3d_bf16(&map, kv, dims, strides, box)) return -1;
   const int threads = (n_cons + 1) * 32;
-  // the cache is streamed with the L2 evict-first policy (SW_XA_EVICT=0: default policy): +1.2 % on the two-lane
-  // bench, measured ABAB on one box (3 796 / 3 851 / 3 809 / 3 844 audio-s/s)
-  static const int evict_first = getenv("SW_XA_EVICT") ? atoi(getenv("SW_XA_EVICT")) : 1;
-  // `ws` holds the partials of THIS call's rows (row0 .. row0 + R) from its start; the main kernel addresses rows
-  // absolutely (through grp_start), so it gets the pointer moved back by row0 rows of n_chunks partials
-  float* ws_main = ws - (int64_t)row0 * n_chunks * (d + 2 * n_head);
 #define XA_LAUNCH(H)                                                                                  \
   do {                                                                                                \
     static SmemOptIn opt_in; /* per device (host_common.h) */                                         \
     SW_CUDA_CHECK(opt_in.ensure(cross_attention_kernel<H>, (int)smem));                               \
     SW_CUDA_CHECK(launch_pdl(cross_attention_kernel<H>, dim3(grid), dim3(threads), smem, stream, map, \
                              q, d_grp_win, d_grp_start, d_grp_count, T, d, n_head, n_cons, spc,        \
-                             n_stages, n_chunks, n_items, ws_main, 0u, n_hsplit, evict_first));        \
+                             n_stages, n_chunks, n_items, ws, 0u, n_hsplit));                         \
   } while (0)
   switch (hpw) {
     case 1: XA_LAUNCH(1); break;
@@ -389,10 +379,8 @@ int cross_attention(const bf16* q, const bf16* kv, int64_t kv_rows, const int* d
   }
 #undef XA_LAUNCH
   if (ev_main_done) SW_CUDA_CHECK(cudaEventRecordWithFlags(ev_main_done, stream, ev_flags));
-  if (ev_dep) SW_CUDA_CHECK(cudaEventRecord(ev_dep, stream));
-  // the main kernel addresses rows through grp_start (absolute); the merge walks this call's rows row0 .. row0 + R
   SW_CUDA_CHECK(launch_pdl(cross_combine_kernel, dim3(R, (n_head + 3) / 4), dim3(32), 0, stream, ws, n_chunks, d, n_head,
-                           out + (int64_t)row0 * d));
+                           out));
   return 0;
 }
 

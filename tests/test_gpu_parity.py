@@ -708,33 +708,3 @@ def test_language_per_utterance_in_one_batch(eng_tiny, ora_tiny):
     with pytest.raises(RuntimeError) as ei:
         eng_tiny.full_batch_pcm16(clips[:2], eng_tiny.default_params(0, **GREEDY), languages=["en", "zz"])
     assert "language" in str(ei.value)
-
-
-def test_interleaved_halves_equal_the_default_step(swb, monkeypatch):
-    """The development lane mode SW_INTERLEAVE=1 (one engine, every decoder step cut into two halves that run as two
-    dependency chains of one CUDA graph with alternating cross attentions) returns what the default step returns:
-    greedy and beam search, ragged batch, halves of unequal size."""
-    from tools import gen_model
-    path, info = model_file("tiny", script_len=40, keyed=4)
-    k = info["keyed"]
-    clips = [synth_audio.keyed_clip(k, synth_audio.keyed_symbols(k, s), seed=s)[: 16000 * n]
-             for s, n in zip(range(500, 507), (30, 30, 12, 30, 7, 30, 21))]
-    outs = []
-    for mode in ("0", "1"):
-        monkeypatch.setenv("SW_INTERLEAVE", mode)
-        monkeypatch.setenv("SW_INTERLEAVE_MIN", "1")
-        e = swb.Engine(path, max_batch=4, max_beams=5, n_lanes=2)
-        assert e.stats()["n_lanes"] == (1 if mode == "1" else 2)
-        outs.append((e.full_batch_pcm16(clips, e.default_params(0, **GREEDY)),
-                     e.full_batch_pcm16(clips[:5], e.default_params(1, language="en", temperature_inc=0.0,
-                                                                    suppress_nst=1, token_timestamps=1, beam_size=5))))
-        e.close()
-    # Whole 30 s clips: everything identical. Cut clips: identical on the prefix their audio decides - behind it the
-    # keyed model's alternatives are near-ties, and the two modes chunk the cross attention differently (the
-    # flash-decoding merge order follows the number of windows of a launch), which may flip a near-tie.
-    for a, b, c in zip(outs[0][0] + outs[0][1], outs[1][0] + outs[1][1], clips + clips[:5]):
-        if len(c) == 16000 * 30:
-            compare_results(a, b)
-        else:
-            sure = gen_model.keyed_sure_prefix(info, len(c))
-            assert sure >= 5 and seg_ids(a)[:sure] == seg_ids(b)[:sure]

@@ -59,24 +59,22 @@ if __name__ == "__main__":
     if len(sys.argv) > 1 and sys.argv[1] == "--case":
         print(json.dumps(one(int(sys.argv[2]))), flush=True)
     elif len(sys.argv) > 1 and sys.argv[1] == "--kernels":
-        # in-chain cost of every kernel beside an occupier that holds 96 SMs, for two skinny ring depths
+        # in-chain cost of every kernel beside an occupier that holds 96 SMs
         names = {0: "chain", 1: "layer_norm x3", 2: "qkv gemm", 4: "self attention", 8: "wo gemm", 16: "wxq gemm",
                  32: "reduce q", 256: "wxo gemm", 512: "fc1 gemm", 1024: "fc2 gemm"}
-        for stages in ("8", "4"):
-            base = None
-            for bit, name in names.items():
-                env = dict(os.environ, SW_SKIP=str(64 | bit), SW_SKINNY_STAGES=stages)
-                out = subprocess.run([sys.executable, __file__, "--case", "1"], env=env, capture_output=True, text=True)
-                try:
-                    r = json.loads(out.stdout.strip().splitlines()[-1])
-                except Exception:
-                    print("skip", bit, "FAILED", out.stdout[-300:], out.stderr[-500:], flush=True)
-                    continue
-                if bit == 0:
-                    base = r["us_per_layer"]
-                r.update(kernel=name, skinny_stages=int(stages),
-                         in_chain_cost_us=None if base is None else round(base - r["us_per_layer"], 2))
-                print(json.dumps(r), flush=True)
+        base = None
+        for bit, name in names.items():
+            env = dict(os.environ, SW_SKIP=str(64 | bit))
+            out = subprocess.run([sys.executable, __file__, "--case", "1"], env=env, capture_output=True, text=True)
+            try:
+                r = json.loads(out.stdout.strip().splitlines()[-1])
+            except Exception:
+                print("skip", bit, "FAILED", out.stdout[-300:], out.stderr[-500:], flush=True)
+                continue
+            if bit == 0:
+                base = r["us_per_layer"]
+            r.update(kernel=name, in_chain_cost_us=None if base is None else round(base - r["us_per_layer"], 2))
+            print(json.dumps(r), flush=True)
     else:
         for ci in range(len(CASES)):
             for skip in ((64, 0, 2047 - 64) if ci == 0 else (64,)):
