@@ -253,6 +253,17 @@ SW_API int sw_dev_skinny_split_k(int kernel, int N, int K);
 SW_API int sw_dev_layer_norm(float* d_x, int rows, int d, const float* g, const float* b,
                              void* d_out_bf16, const float* d_partial, int n_split, const float* d_bias,
                              void* stream);
+/* encoder self attention: qkv [n_win*T][3d] bf16 (Q | K | V), out [n_win*T][d] bf16 */
+SW_API int sw_dev_encoder_attention(const void* d_qkv, void* d_out, int n_win, int T, int d, int n_head, void* stream);
+/* cross attention + combine; ws >= sw_dev_cross_attention_ws_floats(R, d, n_head) floats; max_ctas 0 = one CTA per SM */
+SW_API size_t sw_dev_cross_attention_ws_floats(int R, int d, int n_head);
+SW_API int sw_dev_cross_attention(const void* d_q, const void* d_kv, int64_t kv_rows, const int* d_grp_win,
+                                  const int* d_grp_start, const int* d_grp_count, int n_groups, int max_count, int R,
+                                  int T, int d, int n_head, float* d_ws, void* d_out, int max_ctas, void* stream);
+/* paged causal self attention + append; rows: R DecRow records of 20 int32 each
+   (slot, pos, win, pos0, pages[14], pad[2]); pool [page][n_layer][2][32][d] bf16 */
+SW_API int sw_dev_self_attention(const void* d_qkv, const int* d_rows, int R, int d, int n_head, void* d_pool,
+                                 int layer, int n_layer, void* d_out, void* stream);
 /* development: hold n_ctas SMs (smem_bytes of shared memory and most of the register file each) for ms
    milliseconds on a private stream, optionally streaming stream_bytes of HBM meanwhile; n_ctas <= 0 waits
    for it to leave (tools/dev_chain_occupied.py: cost of a decoder layer's latency chain beside a resident

@@ -132,4 +132,22 @@ int sw_dev_layer_norm(float* d_x, int rows, int d, const float* g, const float* 
   return sw::layer_norm(d_x, rows, d, g, b, static_cast<sw::bf16*>(d_out_bf16), nullptr, d_partial, n_split,
                         (int64_t)rows * d, d_bias, static_cast<cudaStream_t>(stream));
 }
+int sw_dev_encoder_attention(const void* d_qkv, void* d_out, int n_win, int T, int d, int n_head, void* stream) {
+  return sw::encoder_attention_tc(static_cast<const sw::bf16*>(d_qkv), static_cast<sw::bf16*>(d_out), n_win, T, d,
+                                  n_head, static_cast<cudaStream_t>(stream));
+}
+size_t sw_dev_cross_attention_ws_floats(int R, int d, int n_head) { return sw::cross_attention_ws_floats(R, d, n_head); }
+int sw_dev_cross_attention(const void* d_q, const void* d_kv, int64_t kv_rows, const int* d_grp_win,
+                           const int* d_grp_start, const int* d_grp_count, int n_groups, int max_count, int R,
+                           int T, int d, int n_head, float* d_ws, void* d_out, int max_ctas, void* stream) {
+  return sw::cross_attention(static_cast<const sw::bf16*>(d_q), static_cast<const sw::bf16*>(d_kv), kv_rows, d_grp_win,
+                             d_grp_start, d_grp_count, n_groups, max_count, R, T, d, n_head, d_ws,
+                             static_cast<sw::bf16*>(d_out), static_cast<cudaStream_t>(stream), nullptr, 0, max_ctas);
+}
+int sw_dev_self_attention(const void* d_qkv, const int* d_rows, int R, int d, int n_head, void* d_pool,
+                          int layer, int n_layer, void* d_out, void* stream) {
+  return sw::self_attention(static_cast<const sw::bf16*>(d_qkv), reinterpret_cast<const sw::DecRow*>(d_rows), R, d,
+                            n_head, static_cast<sw::bf16*>(d_pool), layer, n_layer, static_cast<sw::bf16*>(d_out),
+                            static_cast<cudaStream_t>(stream));
+}
 }

@@ -86,7 +86,8 @@ EXPORTS = [
     "sw_prosody_default_opts", "sw_prosody_segments_f32", "sw_prosody_segments_pcm16",
     "sw_resample_out_len", "sw_resample_f32",
     "sw_dev_gemm_bf16", "sw_dev_skinny_gemm", "sw_dev_skinny_split", "sw_dev_layer_norm", "sw_dev_occupy",
-    "sw_dev_skinny_gemm_k", "sw_dev_skinny_split_k"]
+    "sw_dev_skinny_gemm_k", "sw_dev_skinny_split_k", "sw_dev_encoder_attention", "sw_dev_cross_attention_ws_floats",
+    "sw_dev_cross_attention", "sw_dev_self_attention"]
 
 _lib = None
 
