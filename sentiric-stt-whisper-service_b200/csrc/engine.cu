@@ -100,13 +100,13 @@ static int engine_init(Engine* e, const char* path, const sw_ctx_params* p, cons
   e->n_pages = (int)(R * KV_MAX_PAGES + R);
   const size_t page_elems = (size_t)hp.n_text_layer * 2 * KV_PAGE * d;
   if (e->kv_pool.alloc((size_t)e->n_pages * page_elems)) return -1;
-  if (e->d_page_table.alloc(R * KV_MAX_PAGES) || e->d_tok.alloc(R) || e->d_pos.alloc(R) ||
+  if (e->d_tok.alloc(R) || e->d_pos.alloc(R) ||
       e->d_grp_win.alloc(R) || e->d_grp_start.alloc(R) || e->d_grp_count.alloc(R) || e->d_rows.alloc(R) ||
       e->d_lrows.alloc(R) || e->d_picks.alloc(R * 8) || e->d_suppress.alloc(hp.n_vocab) ||
       e->d_copy_pairs.alloc(2 * R))
     return -1;
-  if (e->h_page_table.alloc(R * KV_MAX_PAGES) || e->h_tok.alloc(R) || e->h_pos.alloc(R) ||
-      e->h_grp.alloc(3 * R) || e->h_rows.alloc(R) || e->h_lrows.alloc(R) || e->h_picks.alloc(R * 8))
+  if (e->h_tok.alloc(R) || e->h_pos.alloc(R) || e->h_grp.alloc(3 * R) || e->h_rows.alloc(R) ||
+      e->h_lrows.alloc(R) || e->h_picks.alloc(R * 8))
     return -1;
   SW_CUDA_CHECK(cudaDeviceSynchronize());
   {
@@ -237,23 +237,25 @@ int engine_encode(Engine* e, int n_win, float* enc_out_f32) {
 }
 
 int engine_copy_pages(Engine* e, const std::vector<int>& pairs) {
-  if (pairs.empty()) return 0;
   const HParams& hp = e->model->hp;
-  const int n = (int)pairs.size() / 2;
-  SW_CHECK(pairs.size() <= e->d_copy_pairs.n, "too many page copies (%d)", n);
-  // pageable source: the driver stages it before returning, so the vector may die afterwards
-  SW_CUDA_CHECK(cudaMemcpyAsync(e->d_copy_pairs.p, pairs.data(), pairs.size() * sizeof(int),
-                                cudaMemcpyHostToDevice, e->stream));
   const int64_t page_elems = (int64_t)hp.n_text_layer * 2 * KV_PAGE * hp.n_text_state;
-  if (kv_copy_pages(e->kv_pool.p, e->d_copy_pairs.p, n, page_elems, e->stream)) return -1;
-  e->times.n_launches++;
+  // in chunks of what d_copy_pairs holds; each chunk completes before the next overwrites the buffer
+  for (size_t c0 = 0; c0 < pairs.size(); c0 += e->d_copy_pairs.n) {
+    const size_t n = std::min(e->d_copy_pairs.n, pairs.size() - c0);
+    SW_CUDA_CHECK(cudaMemcpyAsync(e->d_copy_pairs.p, pairs.data() + c0, n * sizeof(int), cudaMemcpyHostToDevice,
+                                  e->stream));
+    if (kv_copy_pages(e->kv_pool.p, e->d_copy_pairs.p, (int)n / 2, page_elems, e->stream)) return -1;
+    e->times.n_launches++;
+    SW_CUDA_CHECK(cudaStreamSynchronize(e->stream));
+  }
   return 0;
 }
 
 // Everything one decoder step puts on the stream (uploads, kernels, pick read-back). `launches`
 // counts kernels; `capturing` selects graph-safe event records for the kernel-timing probes.
-static int enqueue_decode_step(Engine* e, int R, int n_groups, int max_count, bool want_logits, int n_lrows,
-                               const LogitCfg& cfg, bool upload_page_table, bool capturing, long* launches) {
+static int enqueue_decode_step(Engine* e, const StepRows& step, bool want_logits, int n_lrows, const LogitCfg& cfg,
+                               bool capturing, long* launches) {
+  const int R = step.R, n_groups = step.G, max_count = step.max_count;
   const Model& m = *e->model;
   const HParams& hp = m.hp;
   const int d = hp.n_text_state, L = hp.n_text_layer;
@@ -342,11 +344,10 @@ static int enqueue_decode_step(Engine* e, int R, int n_groups, int max_count, bo
 // .max_initial_ts) are part of the key. Pointers (d_suppress, the row descriptors) are fixed per lane and
 // their contents are refreshed per run / per step.
 struct StepKey {
-  int R, G, max_count, want_logits, n_lrows, upload_pt, timing, suppress_blank, max_initial_ts_id;
+  int R, G, max_count, want_logits, n_lrows, timing, suppress_blank, max_initial_ts_id;
   bool operator<(const StepKey& o) const {
-    return std::tie(R, G, max_count, want_logits, n_lrows, upload_pt, timing, suppress_blank, max_initial_ts_id) <
-           std::tie(o.R, o.G, o.max_count, o.want_logits, o.n_lrows, o.upload_pt, o.timing, o.suppress_blank,
-                    o.max_initial_ts_id);
+    return std::tie(R, G, max_count, want_logits, n_lrows, timing, suppress_blank, max_initial_ts_id) <
+           std::tie(o.R, o.G, o.max_count, o.want_logits, o.n_lrows, o.timing, o.suppress_blank, o.max_initial_ts_id);
   }
 };
 struct StepGraph {
@@ -366,27 +367,23 @@ static void engine_free_step_graphs(Engine* e) {
   e->step_graphs = nullptr;
 }
 
-int engine_decode_step(Engine* e, int R, int n_groups, int max_count, bool want_logits, int n_lrows,
-                       const LogitCfg& cfg, bool upload_page_table) {
+int engine_decode_step(Engine* e, const StepRows& step, bool want_logits, int n_lrows, const LogitCfg& cfg) {
   const HParams& hp = e->model->hp;
-  const int d = hp.n_text_state, L = hp.n_text_layer;
+  const int d = hp.n_text_state, L = hp.n_text_layer, R = step.R;
   SW_CHECK(R > 0 && R <= e->max_rows, "decode step with %d rows (max %d)", R, e->max_rows);
   cudaStream_t st = e->stream;
-  for (int r = 0; r < R; ++r)  // each row carries its slot's page list (the host table is the pager's)
-    memcpy(e->h_rows.p[r].pages, e->h_page_table.p + (size_t)e->h_rows.p[r].slot * KV_MAX_PAGES,
-           KV_MAX_PAGES * sizeof(int));
+  for (int r = 0; r < R; ++r) e->pager.fill(e->h_rows.p[r].slot, e->h_rows.p[r].pages);
   if (!e->use_graphs) {
     SW_CUDA_CHECK(cudaEventRecord(e->ev0, st));
     long launches = 0;
-    if (enqueue_decode_step(e, R, n_groups, max_count, want_logits, n_lrows, cfg, upload_page_table, false, &launches))
-      return -1;
+    if (enqueue_decode_step(e, step, want_logits, n_lrows, cfg, false, &launches)) return -1;
     e->times.n_launches += launches;
   } else {
     // The step is a fixed launch sequence for a given shape: capture it once per shape and replay
     // it (one host call per step instead of ~460, and no inter-kernel launch gaps).
     if (!e->step_graphs) e->step_graphs = new StepGraphCache();
     StepGraphCache& cache = *static_cast<StepGraphCache*>(e->step_graphs);
-    const StepKey key{R, n_groups, max_count, want_logits ? 1 : 0, n_lrows, 0, e->kernel_timing ? 1 : 0,
+    const StepKey key{R, step.G, step.max_count, want_logits ? 1 : 0, n_lrows, e->kernel_timing ? 1 : 0,
                       cfg.suppress_blank, cfg.max_initial_ts_id};
     auto it = cache.graphs.find(key);
     if (it == cache.graphs.end()) {
@@ -396,8 +393,7 @@ int engine_decode_step(Engine* e, int R, int n_groups, int max_count, bool want_
       }
       StepGraph g;
       SW_CUDA_CHECK(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
-      const int rc = enqueue_decode_step(e, R, n_groups, max_count, want_logits, n_lrows, cfg, upload_page_table,
-                                         true, &g.launches);
+      const int rc = enqueue_decode_step(e, step, want_logits, n_lrows, cfg, true, &g.launches);
       cudaGraph_t graph = nullptr;
       const cudaError_t ce = cudaStreamEndCapture(st, &graph);
       if (rc || ce != cudaSuccess || !graph) {
@@ -431,7 +427,7 @@ int engine_decode_step(Engine* e, int R, int n_groups, int max_count, bool want_
     }
     e->times.n_xattn += n_timed;
     // per launch: the cross-KV of every active window once + q in + attention out
-    e->times.xattn_bytes += (double)n_timed * ((double)n_groups * 1500 * 2 * d * 2 + (double)R * d * 4);
+    e->times.xattn_bytes += (double)n_timed * ((double)step.G * 1500 * 2 * d * 2 + (double)R * d * 4);
   }
   return 0;
 }

@@ -11,6 +11,7 @@
 #include "../../include/sw_whisper.h"
 #include "host_common.h"
 #include "kernels.cuh"
+#include "kv_pager.h"
 #include "model.h"
 
 namespace sw {
@@ -102,13 +103,14 @@ struct Engine {
   DevBuf<bf16> dh, dqkv, datt, dq, dff;
   DevBuf<bf16> kv_pool;
   int n_pages = 0;
-  DevBuf<int> d_page_table, d_tok, d_pos, d_grp_win, d_grp_start, d_grp_count;
+  KvPager pager;                // which kv_pool pages each self-KV slot holds
+  DevBuf<int> d_tok, d_pos, d_grp_win, d_grp_start, d_grp_count;
   DevBuf<DecRow> d_rows;
   DevBuf<LogitRow> d_lrows;
   DevBuf<PickOut> d_picks;
   DevBuf<uint8_t> d_suppress;
   DevBuf<int> d_copy_pairs;
-  PinBuf<int> h_page_table, h_tok, h_pos, h_grp;
+  PinBuf<int> h_tok, h_pos, h_grp;  // step rows: written through StepRows only
   PinBuf<DecRow> h_rows;
   PinBuf<LogitRow> h_lrows;
   PinBuf<PickOut> h_picks;
@@ -132,12 +134,36 @@ Engine* engine_create_lane(const Engine* primary);
 // enc_out_f32 (device, [n_win*1500][d]) may be null.
 int engine_encode(Engine* e, int n_win, float* enc_out_f32);
 
-// one decoder step over R rows (h_rows/h_tok/h_pos filled; rows grouped by window in h_grp).
+// The rows of one decoder step, grouped by window, in the engine's pinned step buffers: per row h_rows, h_tok and
+// h_pos; per group h_grp = window | first row | row count, at stride max_rows. The rows of a group are added
+// between open(win) and close(); engine_decode_step fills their page lists from e->pager.
+struct StepRows {
+  Engine* e;
+  int R = 0, G = 0, max_count = 0;  // rows, groups, most rows in one group
+  explicit StepRows(Engine* eng) : e(eng) {}
+  void open(int win) {
+    e->h_grp.p[G] = win;
+    e->h_grp.p[e->max_rows + G] = R;
+  }
+  // the row of `slot` at position pos; positions pos0..pos of the slot are rows of this step. Returns its index.
+  int add(int slot, int pos, int pos0, int token) {
+    e->h_rows.p[R] = DecRow{slot, pos, e->h_grp.p[G], pos0};
+    e->h_tok.p[R] = token;
+    e->h_pos.p[R] = pos;
+    return R++;
+  }
+  void close() {
+    const int n = R - e->h_grp.p[e->max_rows + G];
+    e->h_grp.p[2 * e->max_rows + G++] = n;
+    max_count = std::max(max_count, n);
+  }
+};
+
+// one decoder step over the rows of `step`.
 // want_logits: final LN + logits GEMM for all rows (e->logits). If n_lrows > 0, h_lrows[0..n_lrows) are
 // processed into h_picks. Synchronises the stream before returning so the host can read them.
-int engine_decode_step(Engine* e, int R, int n_groups, int max_count, bool want_logits, int n_lrows,
-                       const LogitCfg& cfg, bool upload_page_table);
-// device-side copies of whole KV pages (beam reshuffle): pairs [src0, dst0, src1, dst1, ...]
+int engine_decode_step(Engine* e, const StepRows& step, bool want_logits, int n_lrows, const LogitCfg& cfg);
+// device-side copies of whole KV pages: pairs [src0, dst0, src1, dst1, ...], any number of them
 int engine_copy_pages(Engine* e, const std::vector<int>& pairs);
 
 }  // namespace sw

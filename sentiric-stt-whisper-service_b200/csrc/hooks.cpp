@@ -102,20 +102,18 @@ int sw_decode_logits(sw_ctx* ctx, const int32_t* tokens, int n_windows, int n_to
   SW_CHECK(n_tok <= hp.n_text_ctx, "n_tok %d exceeds the text context", n_tok);
   for (int i = 0; i < n_windows * n_tok; ++i)
     SW_CHECK(tokens[i] >= 0 && tokens[i] < hp.n_vocab, "token %d out of range", tokens[i]);
-  for (int w = 0; w < n_windows; ++w)
-    for (int i = 0; i < KV_MAX_PAGES; ++i) e->h_page_table.p[w * KV_MAX_PAGES + i] = w * KV_MAX_PAGES + i;
+  e->pager.reset(e->n_pages, e->max_rows);
   LogitCfg cfg;
   memset(&cfg, 0, sizeof(cfg));
   for (int pos = 0; pos < n_tok; ++pos) {
+    StepRows step(e);
     for (int w = 0; w < n_windows; ++w) {
-      e->h_rows.p[w] = DecRow{w, pos, w, pos};
-      e->h_tok.p[w] = tokens[(size_t)w * n_tok + pos];
-      e->h_pos.p[w] = pos;
-      e->h_grp.p[w] = w;
-      e->h_grp.p[e->max_rows + w] = w;
-      e->h_grp.p[2 * e->max_rows + w] = 1;
+      if (e->pager.ensure(w, pos)) return -1;
+      step.open(w);
+      step.add(w, pos, pos, tokens[(size_t)w * n_tok + pos]);
+      step.close();
     }
-    if (engine_decode_step(e, n_windows, n_windows, 1, true, 0, cfg, pos == 0)) return -1;
+    if (engine_decode_step(e, step, true, 0, cfg)) return -1;
     SW_CUDA_CHECK(cudaMemcpy2DAsync(logits + (size_t)pos * hp.n_vocab, (size_t)n_tok * hp.n_vocab * 4,
                                     e->logits.p, e->logits_ld * 4, (size_t)hp.n_vocab * 4, n_windows,
                                     cudaMemcpyDeviceToHost, e->stream));

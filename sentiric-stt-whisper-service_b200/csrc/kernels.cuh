@@ -91,12 +91,12 @@ constexpr int KV_PAGE = 32;       // tokens per self-KV page
 constexpr int KV_MAX_PAGES = 14;  // 448 / 32
 
 struct DecRow {    // one decoder row of a step
-  int slot;        // self-KV slot (page table row)
+  int slot;        // self-KV slot (whose page list the pager keeps)
   int pos;         // position of this token
   int win;         // window index into the cross-KV batch
   int pos0;        // first position of this slot whose K/V is produced in this very step: positions
                    // pos0..pos come from rows r-(pos-pos0)..r of the step (contiguous), older ones from the cache
-  int pages[KV_MAX_PAGES];  // the slot's page list (filled by engine_decode_step from the host page table):
+  int pages[KV_MAX_PAGES];  // the slot's page list (filled by engine_decode_step from the host pager):
                             // the attention kernel needs no second dependent lookup
   int pad[2];
 };

@@ -71,58 +71,6 @@ struct Window {  // one job in flight
   std::vector<int> tt_segs;  // result segments this window emitted whose token times still need the energy pass
 };
 
-// ---- paged self-KV bookkeeping (host): page tables with reference counts ------------------
-struct Pager {
-  int n_pages = 0, n_slots = 0;
-  std::vector<int> refc, free_list;
-  int* table = nullptr;  // [n_slots][KV_MAX_PAGES], pinned, mirrors the device copy
-  bool dirty = true;
-  void reset(int pages, int slots, int* tbl) {
-    n_pages = pages;
-    n_slots = slots;
-    table = tbl;
-    refc.assign(pages, 0);
-    free_list.resize(pages);
-    for (int i = 0; i < pages; ++i) free_list[i] = pages - 1 - i;
-    std::fill(table, table + (size_t)slots * KV_MAX_PAGES, 0);
-    owned.assign((size_t)slots * KV_MAX_PAGES, -1);
-    dirty = true;
-  }
-  std::vector<int> owned;  // page id or -1
-  int alloc() {
-    if (free_list.empty()) return -1;
-    const int p = free_list.back();
-    free_list.pop_back();
-    refc[p] = 1;
-    return p;
-  }
-  void unref(int p) {
-    if (p >= 0 && --refc[p] == 0) free_list.push_back(p);
-  }
-  int& at(int slot, int i) { return owned[(size_t)slot * KV_MAX_PAGES + i]; }
-  void set(int slot, int i, int page) {
-    at(slot, i) = page;
-    table[(size_t)slot * KV_MAX_PAGES + i] = page < 0 ? 0 : page;
-    dirty = true;
-  }
-  // make sure `slot` can write position pos
-  int ensure(int slot, int pos) {
-    const int i = pos / KV_PAGE;
-    if (at(slot, i) >= 0) return 0;
-    const int p = alloc();
-    if (p < 0) return -1;
-    set(slot, i, p);
-    return 0;
-  }
-  void release_slot(int slot) {
-    for (int i = 0; i < KV_MAX_PAGES; ++i)
-      if (at(slot, i) >= 0) {
-        unref(at(slot, i));
-        set(slot, i, -1);
-      }
-  }
-};
-
 // whisper_sequence_score
 void sequence_score(const sw_full_params& p, Sequence& s) {
   if (s.result_len == 0) return;
@@ -273,7 +221,6 @@ struct Run {
   std::vector<float> temps;
   std::vector<int> prompt_init_tail;  // [transcribe|translate] (+ [not])
   LogitCfg cfg;
-  Pager pager;
   int beam = 1, best_of = 1;
   Run(Engine* e_, const sw_full_params& p_) : e(e_), p(p_), m(*e_->model) {}
 
@@ -431,17 +378,15 @@ struct Run {
       std::vector<int> wutt(need.begin() + b0, need.begin() + b0 + nb), wseek(nb, 0);
       if (finalize_windows(wutt, wseek)) return -1;
       if (engine_encode(e, nb, nullptr)) return -1;
-      pager.reset(e->n_pages, e->max_rows, e->h_page_table.p);
+      e->pager.reset(e->n_pages, e->max_rows);
+      StepRows step(e);
       for (int w = 0; w < nb; ++w) {
-        if (pager.ensure(w, 0)) return -1;
-        e->h_rows.p[w] = DecRow{w, 0, w, 0};
-        e->h_tok.p[w] = v.sot;
-        e->h_pos.p[w] = 0;
-        e->h_grp.p[w] = w;
-        e->h_grp.p[e->max_rows + w] = w;
-        e->h_grp.p[2 * e->max_rows + w] = 1;
+        if (e->pager.ensure(w, 0)) return -1;
+        step.open(w);
+        step.add(w, 0, 0, v.sot);
+        step.close();
       }
-      if (engine_decode_step(e, nb, nb, 1, true, 0, cfg, true)) return -1;
+      if (engine_decode_step(e, step, true, 0, cfg)) return -1;
       std::vector<float> lg((size_t)nb * v.n_langs);
       SW_CUDA_CHECK(cudaMemcpy2DAsync(lg.data(), v.n_langs * sizeof(float), e->logits.p + v.sot + 1,
                                       e->logits_ld * sizeof(float), v.n_langs * sizeof(float), nb,
@@ -529,162 +474,157 @@ struct Run {
     if (i == n_max - 1 && (d.seq.result_len == 0 || d.seek_delta < CHUNK_CS / 2)) d.failed = true;
   }
 
-  // ---- decode a batch of windows to completion; cross-KV for window index w is already in place
-  int decode_windows(std::vector<Window>& wins) {
-    const int nw = (int)wins.size(), MR = e->max_rows;
-    // self-KV slots: window w owns slots [slot_base[w], slot_base[w] + n_cur) - the batch was admitted with
-    // sum(n_cur) <= MR rows, so every slot index stays below the page table's MR rows
-    std::vector<int> slot_base(nw, 0);
-    for (int w = 1; w < nw; ++w) slot_base[w] = slot_base[w - 1] + wins[w - 1].n_cur;
-    const int n_max = m.hp.n_text_ctx / 2 - 4;
-    pager.reset(e->n_pages, MR, e->h_page_table.p);
-    auto slot_of = [&](int w, int j) { return slot_base[w] + j; };
+  using Picks = std::vector<std::vector<std::vector<PickOut>>>;  // [window][decoder][draw] of the last step
 
-    // ---- prompts, position by position (only decoder 0 of each window)
-    int max_prompt = 0;
-    for (auto& w : wins) max_prompt = std::max(max_prompt, (int)w.prompt.size());
-    std::vector<int> prompt_row(nw, -1);
-    int total_prompt_rows = 0;
-    for (auto& w : wins) total_prompt_rows += (int)w.prompt.size();
-    // Common case ([sot, lang, task]): every prompt position of every window in ONE step - the rows
-    // of a window share its cross-KV read (they sit in the M dimension of the cross-attention MMAs)
-    // and self attention is causal over the positions appended in the same step.
-    const bool one_step = total_prompt_rows <= MR && max_prompt <= 8;
-    if (one_step) {
-      int R = 0, G = 0, n_lr = 0, max_cnt = 1;
-      std::vector<std::pair<int, int>> lmap;
-      for (int wi = 0; wi < nw; ++wi) {
-        Window& w = wins[wi];
-        const int s = slot_of(wi, 0), start = R, P = (int)w.prompt.size();
-        for (int pos = 0; pos < P; ++pos) {
-          if (pager.ensure(s, pos)) {
-            set_last_error("self-KV page pool exhausted");
-            return -1;
-          }
-          e->h_rows.p[R] = DecRow{s, pos, wi, 0};  // positions 0..pos of this slot are all rows of this step
-          e->h_tok.p[R] = w.prompt[pos];
-          e->h_pos.p[R] = pos;
-          ++R;
-        }
-        prompt_row[wi] = R - 1;
-        e->h_grp.p[G] = wi;
-        e->h_grp.p[MR + G] = start;
-        e->h_grp.p[2 * MR + G] = P;
-        max_cnt = std::max(max_cnt, P);
-        ++G;
-      }
-      for (int wi = 0; wi < nw; ++wi)
-        for (int j = 0; j < wins[wi].n_cur && n_lr < MR; ++j) {
-          fill_lrow(e->h_lrows.p[n_lr], wins[wi], j, prompt_row[wi], true);
-          lmap.push_back({wi, j});
-          ++n_lr;
-        }
-      if (engine_decode_step(e, R, G, max_cnt, true, n_lr, cfg, pager.dirty)) return -1;
-      pager.dirty = false;
-      for (auto& w : wins) utts[w.utt].res->n_decode_steps++;
-      for (int k = 0; k < n_lr; ++k) first_picks.push_back({lmap[k].first, lmap[k].second, k});
-      for (int k = 0; k < n_lr; ++k)
-        for (int q = 0; q < 8; ++q) first_store.push_back(e->h_picks.p[k * 8 + q]);
+  // ---- the prompt of every window into the self-KV of its first slot; the step in which a window's prompt ends
+  // gives each of its decoders its first distribution. Common case ([sot, lang, task]): every position in ONE step -
+  // the rows of a window share its cross-KV read (they sit in the M dimension of the cross-attention MMAs, which take
+  // up to 8 rows per window) and self attention is causal over the positions appended in the same step. Longer
+  // prompts go one position per step.
+  int prefill(std::vector<Window>& wins, const std::vector<int>& slot0, Picks& picks) {
+    int max_prompt = 0, total = 0;
+    for (auto& w : wins) {
+      max_prompt = std::max(max_prompt, (int)w.prompt.size());
+      total += (int)w.prompt.size();
     }
-    for (int pos = 0; pos < max_prompt && !one_step; ++pos) {
-      int R = 0, G = 0, n_lr = 0;
-      for (int wi = 0; wi < nw; ++wi) {
+    const int chunk = total <= e->max_rows && max_prompt <= 8 ? max_prompt : 1;
+    for (int pos0 = 0; pos0 < max_prompt; pos0 += chunk) {
+      StepRows step(e);
+      std::vector<std::pair<int, int>> lmap;  // (window, decoder) of each logit row
+      for (int wi = 0; wi < (int)wins.size(); ++wi) {
         Window& w = wins[wi];
-        if (pos >= (int)w.prompt.size()) continue;
-        const int s = slot_of(wi, 0);
-        if (pager.ensure(s, pos)) {
-          set_last_error("self-KV page pool exhausted");
-          return -1;
+        const int P = (int)w.prompt.size(), end = std::min(P, pos0 + chunk);
+        if (pos0 >= P) continue;
+        int row = 0;
+        step.open(wi);
+        for (int pos = pos0; pos < end; ++pos) {
+          if (e->pager.ensure(slot0[wi], pos)) return -1;
+          row = step.add(slot0[wi], pos, pos0, w.prompt[pos]);
         }
-        e->h_rows.p[R] = DecRow{s, pos, wi, pos};
-        e->h_tok.p[R] = w.prompt[pos];
-        e->h_pos.p[R] = pos;
-        e->h_grp.p[G] = wi;
-        e->h_grp.p[MR + G] = R;
-        e->h_grp.p[2 * MR + G] = 1;
-        if (pos == (int)w.prompt.size() - 1) prompt_row[wi] = R;
-        ++R;
-        ++G;
-      }
-      // rows whose prompt ends here get their first distribution
-      std::vector<std::pair<int, int>> lmap;  // (window, decoder)
-      for (int wi = 0; wi < nw; ++wi) {
-        Window& w = wins[wi];
-        if (pos != (int)w.prompt.size() - 1) continue;
+        step.close();
+        if (end < P) continue;
         for (int j = 0; j < w.n_cur; ++j) {
-          fill_lrow(e->h_lrows.p[n_lr], w, j, prompt_row[wi], true);
+          fill_lrow(e->h_lrows.p[lmap.size()], w, j, row, true);
           lmap.push_back({wi, j});
-          ++n_lr;
         }
+        utts[w.utt].res->n_decode_steps++;
       }
-      if (engine_decode_step(e, R, G, 1, n_lr > 0, n_lr, cfg, pager.dirty)) return -1;
-      pager.dirty = false;
-      for (auto& w : wins)
-        if (pos == (int)w.prompt.size() - 1) utts[w.utt].res->n_decode_steps++;
-      const int base = (int)first_store.size() / 8;
-      for (int k = 0; k < n_lr; ++k) first_picks.push_back({lmap[k].first, lmap[k].second, base + k});
-      // keep the picks: h_picks is overwritten by the next step
+      const int n_lr = (int)lmap.size();
+      if (engine_decode_step(e, step, n_lr > 0, n_lr, cfg)) return -1;
       for (int k = 0; k < n_lr; ++k)
-        for (int q = 0; q < 8; ++q) first_store.push_back(e->h_picks.p[k * 8 + q]);
+        std::copy_n(e->h_picks.p + k * 8, 8, picks[lmap[k].first][lmap[k].second].begin());
     }
-    // share the prompt KV with decoders 1..n_cur-1 (prompt pages are private copies: the last
-    // page is partial and will be written by every decoder)
-    {
-      std::vector<int> pairs;
-      for (int wi = 0; wi < nw; ++wi) {
-        Window& w = wins[wi];
-        const int np = ((int)w.prompt.size() + KV_PAGE - 1) / KV_PAGE;
-        for (int j = 1; j < w.n_cur; ++j)
-          for (int pi = 0; pi < np; ++pi) {
-            const int src = pager.at(slot_of(wi, 0), pi);
-            const bool full = (pi + 1) * KV_PAGE <= (int)w.prompt.size();
-            if (full) {
-              pager.refc[src]++;
-              pager.set(slot_of(wi, j), pi, src);
-            } else {
-              const int np2 = pager.alloc();
-              if (np2 < 0) {
-                set_last_error("self-KV page pool exhausted");
-                return -1;
-              }
-              pager.set(slot_of(wi, j), pi, np2);
-              pairs.push_back(src);
-              pairs.push_back(np2);
-            }
-          }
-      }
-      for (size_t c0 = 0; c0 < pairs.size(); c0 += 2 * (size_t)MR) {
-        std::vector<int> part(pairs.begin() + c0, pairs.begin() + std::min(pairs.size(), c0 + 2 * (size_t)MR));
-        if (engine_copy_pages(e, part)) return -1;
-        SW_CUDA_CHECK(cudaStreamSynchronize(e->stream));
-      }
-    }
-    // picks for iteration 0, indexed [window][decoder][draw]
-    std::vector<std::vector<std::vector<PickOut>>> picks(nw);
-    for (int wi = 0; wi < nw; ++wi) picks[wi].assign(wins[wi].n_cur, std::vector<PickOut>(8));
-    for (auto& fp : first_picks)
-      for (int q = 0; q < 8; ++q) picks[fp.w][fp.j][q] = first_store[(size_t)fp.k_global * 8 + q];
-    first_picks.clear();
-    first_store.clear();
-    for (int wi = 0; wi < nw; ++wi) wins[wi].no_speech_prob = picks[wi][0][0].no_speech_prob;
+    return 0;
+  }
 
+  // ---- beam search over one window at iteration i: the decoders continue the best distinct candidates among
+  // beam draws of each, and positions [0, prompt + i) of the self-KV follow each candidate's source decoder
+  int select_beams(Window& w, const std::vector<std::vector<PickOut>>& wp, int i, int slot0, std::vector<int>& copies,
+                   std::vector<int>& release) {
     struct Cand {
       int decoder_idx, seek_delta;
       bool has_ts;
       Sequence seq;
     };
+    std::vector<Cand> cands;
+    for (int j = 0; j < w.n_cur; ++j) {
+      Decoder& d = w.dec[j];
+      if (d.completed || d.failed) continue;
+      for (int k = 0; k < beam; ++k) {
+        Cand c{j, d.seek_delta, d.has_ts, d.seq};
+        const sw_token_data t = to_token(wp[j][k]);
+        c.seq.tokens.push_back(t);
+        c.seq.sum_logprobs_all += t.plog;
+        cands.push_back(std::move(c));
+      }
+    }
+    std::stable_sort(cands.begin(), cands.end(), [](const Cand& a, const Cand& b) {
+      if (a.seq.sum_logprobs_all != b.seq.sum_logprobs_all) return a.seq.sum_logprobs_all > b.seq.sum_logprobs_all;
+      return a.decoder_idx < b.decoder_idx;
+    });
+    size_t cc = 0;
+    std::vector<int> src(w.n_cur, -1);
+    for (int j = 0; j < w.n_cur; ++j) {
+      Decoder& d = w.dec[j];
+      if (d.completed || d.failed) continue;
+      if (cc >= cands.size()) cc = 0;
+      Cand& cur = cands[cc++];
+      while (cands.size() > cc && same_tokens(cands[cc].seq, cur.seq) && i > 0) ++cc;
+      d.seek_delta = cur.seek_delta;
+      d.has_ts = cur.has_ts;
+      d.seq = cur.seq;
+      src[j] = cur.decoder_idx;
+    }
+    return e->pager.remap(slot0, src, (int)w.prompt.size() + i, copies, release);
+  }
+
+  // ---- the step at position prompt + i: one row per active decoder, grouped by window; its picks go to `picks`
+  int next_step(std::vector<Window>& wins, const std::vector<int>& slot0, int i, Picks& picks) {
+    StepRows step(e);
+    std::vector<std::pair<int, int>> rmap;  // (window, decoder) of each row
+    double kv_tokens = 0;                   // self-KV positions the rows read
+    for (int wi = 0; wi < (int)wins.size(); ++wi) {
+      Window& w = wins[wi];
+      if (w.done) continue;
+      const int pos = (int)w.prompt.size() + i;
+      step.open(wi);
+      for (int j = 0; j < w.n_cur; ++j) {
+        Decoder& d = w.dec[j];
+        if (d.completed || d.failed) continue;
+        if (e->pager.ensure(slot0[wi] + j, pos)) return -1;
+        const int row = step.add(slot0[wi] + j, pos, pos, d.seq.tokens.back().id);
+        fill_lrow(e->h_lrows.p[row], w, j, row, false);
+        rmap.push_back({wi, j});
+        kv_tokens += pos + 1;
+      }
+      step.close();
+      utts[w.utt].res->n_decode_steps++;
+    }
+    if (engine_decode_step(e, step, true, step.R, cfg)) return -1;
+    for (int k = 0; k < step.R; ++k)
+      std::copy_n(e->h_picks.p + k * 8, 8, picks[rmap[k].first][rmap[k].second].begin());
+    // decode-step byte accounting (roofline): weights + per-window cross-KV + self-KV read
+    const double L = m.hp.n_text_layer, dd = m.hp.n_text_state;
+    e->times.decode_bytes +=
+        (double)m.weight_bytes_decoder + step.G * L * 2.0 * 1500 * dd * 2.0 + L * 2.0 * dd * 2.0 * kv_tokens;
+    return 0;
+  }
+
+  // ---- decode a batch of windows to completion; cross-KV for window index w is already in place
+  int decode_windows(std::vector<Window>& wins) {
+    const int nw = (int)wins.size();
+    // self-KV slots: window w owns slots [slot0[w], slot0[w] + n_cur) - the batch was admitted with
+    // sum(n_cur) <= max_rows rows, so every slot index stays below the pager's max_rows slots
+    std::vector<int> slot0(nw, 0);
+    for (int w = 1; w < nw; ++w) slot0[w] = slot0[w - 1] + wins[w - 1].n_cur;
+    e->pager.reset(e->n_pages, e->max_rows);
+    Picks picks(nw);
+    for (int wi = 0; wi < nw; ++wi) picks[wi].assign(wins[wi].n_cur, std::vector<PickOut>(8));
+    if (prefill(wins, slot0, picks)) return -1;
+    for (int wi = 0; wi < nw; ++wi) wins[wi].no_speech_prob = picks[wi][0][0].no_speech_prob;
+    // every decoder of a window starts from the prompt KV of its first
+    std::vector<int> copies, release;
+    for (int wi = 0; wi < nw; ++wi)
+      if (e->pager.remap(slot0[wi], std::vector<int>(wins[wi].n_cur, 0), (int)wins[wi].prompt.size(), copies,
+                         release))
+        return -1;
+    if (engine_copy_pages(e, copies)) return -1;
+    e->pager.unref(release);
+    const int n_max = m.hp.n_text_ctx / 2 - 4;
     for (int i = 0; i < n_max; ++i) {
       if (aborted()) {
         set_last_error("aborted by callback");
         return -6;
       }
-      std::vector<int> copy_pairs;
+      copies.clear();
+      release.clear();
       bool any_active = false;
       for (int wi = 0; wi < nw; ++wi) {
         Window& w = wins[wi];
         if (w.done) continue;
-        const bool beam_mode = p.strategy == 1;
-        if (!beam_mode) {
+        if (p.strategy == 1) {
+          if (select_beams(w, picks[wi], i, slot0[wi], copies, release)) return -1;
+        } else {
           for (int j = 0; j < w.n_cur; ++j) {
             Decoder& d = w.dec[j];
             if (d.completed || d.failed) continue;
@@ -692,89 +632,7 @@ struct Run {
             d.seq.tokens.push_back(t);
             d.seq.sum_logprobs_all += t.plog;
           }
-        } else {
-          std::vector<Cand> cands;
-          for (int j = 0; j < w.n_cur; ++j) {
-            Decoder& d = w.dec[j];
-            if (d.completed || d.failed) continue;
-            for (int k = 0; k < beam; ++k) {
-              Cand c{j, d.seek_delta, d.has_ts, d.seq};
-              const sw_token_data t = to_token(picks[wi][j][k]);
-              c.seq.tokens.push_back(t);
-              c.seq.sum_logprobs_all += t.plog;
-              cands.push_back(std::move(c));
-            }
-          }
-          std::stable_sort(cands.begin(), cands.end(), [](const Cand& a, const Cand& b) {
-            if (a.seq.sum_logprobs_all != b.seq.sum_logprobs_all)
-              return a.seq.sum_logprobs_all > b.seq.sum_logprobs_all;
-            return a.decoder_idx < b.decoder_idx;
-          });
-          size_t cc = 0;
-          std::vector<int> src(w.n_cur, -1);
-          for (int j = 0; j < w.n_cur; ++j) {
-            Decoder& d = w.dec[j];
-            if (d.completed || d.failed) continue;
-            if (cc >= cands.size()) cc = 0;
-            Cand& cur = cands[cc++];
-            while (cands.size() > cc && same_tokens(cands[cc].seq, cur.seq) && i > 0) ++cc;
-            d.seek_delta = cur.seek_delta;
-            d.has_ts = cur.has_ts;
-            d.seq = cur.seq;
-            src[j] = cur.decoder_idx;
-          }
-          // KV reshuffle on page tables: positions [0, n_kv) of decoder src[j] become decoder j's
-          const int n_kv = (int)w.prompt.size() + i;
-          const int np = (n_kv + KV_PAGE - 1) / KV_PAGE;
-          std::vector<std::vector<int>> newtab(w.n_cur);
-          std::vector<int> moved(w.n_cur, 0);  // partial page of source s already handed over
-          for (int j = 0; j < w.n_cur; ++j) {
-            if (src[j] < 0) continue;
-            newtab[j].assign(np, -1);
-            for (int pi = 0; pi < np; ++pi) {
-              const int sp = pager.at(slot_of(wi, src[j]), pi);
-              const bool full = (pi + 1) * KV_PAGE <= n_kv;
-              if (full) {
-                pager.refc[sp]++;
-                newtab[j][pi] = sp;
-              } else if (!moved[src[j]] && src[j] == j) {
-                pager.refc[sp]++;
-                newtab[j][pi] = sp;
-                moved[src[j]] = 1;
-              } else {
-                newtab[j][pi] = -2;  // needs a private copy of sp
-              }
-            }
-          }
-          for (int j = 0; j < w.n_cur; ++j) {
-            if (src[j] < 0) continue;
-            for (int pi = 0; pi < np; ++pi)
-              if (newtab[j][pi] == -2) {
-                const int sp = pager.at(slot_of(wi, src[j]), pi);
-                const int fresh = pager.alloc();
-                if (fresh < 0) {
-                  set_last_error("self-KV page pool exhausted");
-                  return -1;
-                }
-                newtab[j][pi] = fresh;
-                copy_pairs.push_back(sp);
-                copy_pairs.push_back(fresh);
-              }
-          }
-          // sources must stay alive until the copies are enqueued: release after building all tables
-          std::vector<int> to_unref;
-          for (int j = 0; j < w.n_cur; ++j) {
-            if (src[j] < 0) continue;
-            for (int pi = 0; pi < KV_MAX_PAGES; ++pi)
-              if (pager.at(slot_of(wi, j), pi) >= 0) to_unref.push_back(pager.at(slot_of(wi, j), pi));
-          }
-          for (int j = 0; j < w.n_cur; ++j) {
-            if (src[j] < 0) continue;
-            for (int pi = 0; pi < KV_MAX_PAGES; ++pi) pager.set(slot_of(wi, j), pi, pi < np ? newtab[j][pi] : -1);
-          }
-          deferred_unref.insert(deferred_unref.end(), to_unref.begin(), to_unref.end());
         }
-        // state update
         bool all_done = true;
         for (int j = 0; j < w.n_cur; ++j) {
           Decoder& d = w.dec[j];
@@ -785,68 +643,13 @@ struct Run {
         w.done = all_done;
         if (!all_done) any_active = true;
       }
-      if (!copy_pairs.empty()) {
-        for (size_t c0 = 0; c0 < copy_pairs.size(); c0 += 2 * (size_t)MR) {
-          std::vector<int> part(copy_pairs.begin() + c0,
-                                copy_pairs.begin() + std::min(copy_pairs.size(), c0 + 2 * (size_t)MR));
-          if (engine_copy_pages(e, part)) return -1;
-          SW_CUDA_CHECK(cudaStreamSynchronize(e->stream));
-        }
-      }
-      for (int pg : deferred_unref) pager.unref(pg);
-      deferred_unref.clear();
+      if (engine_copy_pages(e, copies)) return -1;
+      e->pager.unref(release);
       if (!any_active) break;
-
-      // ---- next step: one row per active decoder, grouped by window
-      int R = 0, G = 0, max_cnt = 1, n_lr = 0;
-      std::vector<std::pair<int, int>> rmap;
-      for (int wi = 0; wi < nw; ++wi) {
-        Window& w = wins[wi];
-        if (w.done) continue;
-        const int start = R;
-        for (int j = 0; j < w.n_cur; ++j) {
-          Decoder& d = w.dec[j];
-          if (d.completed || d.failed) continue;
-          const int s = slot_of(wi, j), pos = (int)w.prompt.size() + i;
-          if (pager.ensure(s, pos)) {
-            set_last_error("self-KV page pool exhausted");
-            return -1;
-          }
-          e->h_rows.p[R] = DecRow{s, pos, wi, pos};
-          e->h_tok.p[R] = d.seq.tokens.back().id;
-          e->h_pos.p[R] = pos;
-          fill_lrow(e->h_lrows.p[n_lr], w, j, R, false);
-          rmap.push_back({wi, j});
-          ++n_lr;
-          ++R;
-        }
-        e->h_grp.p[G] = wi;
-        e->h_grp.p[MR + G] = start;
-        e->h_grp.p[2 * MR + G] = R - start;
-        max_cnt = std::max(max_cnt, R - start);
-        ++G;
-        utts[w.utt].res->n_decode_steps++;
-      }
-      if (engine_decode_step(e, R, G, max_cnt, true, n_lr, cfg, pager.dirty)) return -1;
-      pager.dirty = false;
-      for (int k = 0; k < n_lr; ++k)
-        for (int q = 0; q < 8; ++q) picks[rmap[k].first][rmap[k].second][q] = e->h_picks.p[k * 8 + q];
-      // decode-step byte accounting (roofline): weights + per-window cross-KV + self-KV read
-      {
-        const double dd = m.hp.n_text_state;
-        double bytes = (double)m.weight_bytes_decoder + (double)G * m.hp.n_text_layer * 2.0 * 1500 * dd * 2.0;
-        for (int k = 0; k < R; ++k) bytes += (double)m.hp.n_text_layer * 2.0 * dd * 2.0 * (e->h_pos.p[k] + 1);
-        e->times.decode_bytes += bytes;
-      }
+      if (next_step(wins, slot0, i, picks)) return -1;
     }
     return 0;
   }
-  struct FirstPick {
-    int w, j, k_global;
-  };
-  std::vector<FirstPick> first_picks;
-  std::vector<PickOut> first_store;
-  std::vector<int> deferred_unref;
 
   // ---- second half of the token-level timestamps for every segment the windows of a finished batch emitted:
   // token times up, one kernel over the energy that never left the device, token times back (token_times.cu).
@@ -1037,9 +840,8 @@ struct Run {
     w.done = false;
   }
 
-  int run(const void* const* pcm, const int* n_samples, int n, bool is_f32, sw_result** out,
-          const char* const* langs) {
-    const Vocab& v = m.vocab;
+  // ---- decoders per window and the temperature ladder
+  int setup_decoding() {
     beam = p.strategy == 1 ? std::max(1, p.beam_size) : 1;
     best_of = std::max(1, p.best_of);
     if (p.strategy == 1) best_of = std::max(1, p.best_of);  // upstream: used when falling back to t > 0
@@ -1053,16 +855,12 @@ struct Run {
       for (float t = p.temperature; t < 1.0f + 1e-6f; t += p.temperature_inc) temps.push_back(t);
     else
       temps.push_back(p.temperature);
-    for (int i = 0; i < n; ++i) SW_CHECK(n_samples[i] >= 0 && (n_samples[i] == 0 || pcm[i]), "utterance %d: null PCM", i);
-    const bool trace = getenv("SW_TRACE") != nullptr;
-    const double tf0 = wall_ms();
-    if (setup_logit_cfg()) return -1;
-    if (front_end(pcm, n_samples, n, is_f32)) return -1;
-    if (trace) fprintf(stderr, "[sw trace] front end of %d utterances: %.1f ms (wall)\n", n, wall_ms() - tf0);
-    for (int i = 0; i < n; ++i) {
-      out[i] = new sw_result();
-      utts[i].res = out[i];
-    }
+    return 0;
+  }
+
+  // ---- per utterance: its language (given, or detected on its first window), the initial prompt and its first job
+  int plan_utterances(int n, const char* const* langs, std::deque<Job>& queue) {
+    const Vocab& v = m.vocab;
     // language
     std::vector<int> need;
     for (int i = 0; i < n; ++i) {
@@ -1088,7 +886,6 @@ struct Run {
       init_prompt = tokenize(m, p.initial_prompt);
     for (int t : init_prompt) SW_CHECK(t >= 0 && t < m.hp.n_vocab, "prompt token %d out of range", t);
 
-    std::deque<Job> queue;
     for (int i = 0; i < n; ++i) {
       Utt& u = utts[i];
       u.res->lang_id = u.lang;
@@ -1099,6 +896,24 @@ struct Run {
       if (u.seek + 100 >= u.seek_end) continue;
       queue.push_back(Job{i, 0});
     }
+    return 0;
+  }
+
+  int run(const void* const* pcm, const int* n_samples, int n, bool is_f32, sw_result** out,
+          const char* const* langs) {
+    if (setup_decoding()) return -1;
+    for (int i = 0; i < n; ++i) SW_CHECK(n_samples[i] >= 0 && (n_samples[i] == 0 || pcm[i]), "utterance %d: null PCM", i);
+    const bool trace = getenv("SW_TRACE") != nullptr;
+    const double tf0 = wall_ms();
+    if (setup_logit_cfg()) return -1;
+    if (front_end(pcm, n_samples, n, is_f32)) return -1;
+    if (trace) fprintf(stderr, "[sw trace] front end of %d utterances: %.1f ms (wall)\n", n, wall_ms() - tf0);
+    for (int i = 0; i < n; ++i) {
+      out[i] = new sw_result();
+      utts[i].res = out[i];
+    }
+    std::deque<Job> queue;
+    if (plan_utterances(n, langs, queue)) return -1;
     // Host post-processing of a finished batch (ranking, segments, token-level timestamps) runs on
     // worker threads while the GPU already encodes / decodes the next batch of other utterances.
     struct Pending {
